@@ -23,6 +23,10 @@ ImageDetect:detect + Tester_FRCNN:testOne do per image.
             engine issues 3 bf16 MMAs per algorithmic MAC (bf16x3 fp32 emulation); `issued_frac` = 3x.
 `cpu_baseline`: the CPU oracle port (torch-CPU fp32 dense layers + C restatement + literal nms.c) timed
             on the box's host cores on one image of the same workload (rank 0, N=1 only).
+`--dump-outputs DIR`: after the run, rank 0 writes what the last step of the `value` loop returned, as float32 .npy files:
+            scores (R x C), bboxes (R x 4C), keep ((C-1) x R proposal rows in NMS emission order, -1 past keep_count),
+            keep_count (C-1) and detections (the gathered records of every rank's last image, N x MPN_REC_FLOATS). The inputs
+            are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -284,15 +288,9 @@ def run_reference(args, rank, world):
         G.test_one(spec, img, boxes, 1.0, W, H, -1.5, 0.3, nms_fn=nms_fn)
         return time.perf_counter() - t0
 
-    # bounded run: one full image costs seconds on the host cores, so at most ~150 s of timed work (and one warm-up image)
-    # whatever --steps/--warmup say; `steps_timed` is what was actually measured
+    # one full image costs about a second on the host cores: one warm-up image whatever --warmup says, then --steps images
     t_first = step(0) if args.warmup > 0 else None
-    budget_s = 150.0
-    ts = []
-    for i in range(args.steps):
-        if ts and sum(ts) + ts[-1] > budget_s:
-            break
-        ts.append(step(1 + i))
+    ts = [step(1 + i) for i in range(args.steps)]
     total = sum(ts)
     val = R * len(ts) / total
     line = {"impl": "reference", "metric": "proposals/sec", "value": val, "unit": "proposals/s", "n_gpus": args.gpus,
@@ -311,19 +309,24 @@ def run_reference(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; 3 with --impl reference)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default 5; 1 with --impl reference)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--replicas", type=int, default=2, help="model replicas per GPU, each on its own mpn_ctx / stream (images dealt round-robin)")
     ap.add_argument("--config", default="vgg16_frcnn", choices=list(WORKLOADS) + ["nms_sweep"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "nms_sweep"):
+        ap.error("--dump-outputs writes the outputs of the GPU arm's detection workloads")
+    if args.steps is None:
+        args.steps = 3 if args.impl == "reference" else 200       # the CPU arm's defaults are sized for a run of a few minutes
+    if args.warmup is None:
+        args.warmup = 1 if args.impl == "reference" else 5
     global H, W, R, C, WORKLOAD
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
-        if args.steps == 200 and args.warmup == 5:
-            args.steps, args.warmup = 3, 1         # defaults sized for a CPU run of a few minutes
         return run_reference(args, rank, world)
 
     if args.config == "nms_sweep":
@@ -446,10 +449,16 @@ def main():
     det_counts = np.array([[g[r, i % K, i // K, 0] for i in range(args.steps)] for r in range(world)])
     assert np.array_equal(g[rank], records_d.cpu().numpy()), "gathered records differ from this rank's own"
     assert det_counts.min() >= 1 and det_counts.max() <= mpn.MPN_MAX_DET, "gathered detection records are empty or overflowed"
+    dump = None
+    if args.dump_outputs and rank == 0:             # the last step's buffers, before the loops below overwrite them
+        last = args.steps - 1
+        sc, bb, kp, ct = (x.cpu().numpy() for x in outs_d[last % K])
+        dump = {"scores": sc, "bboxes": bb, "keep": np.where(np.arange(R) < ct[:, None], kp, -1), "keep_count": ct,
+                "detections": g[:, last % K, last // K]}
 
-    # ---- p50 latency of ONE image on ONE replica over a fixed >= 200-image loop (SURVEY 8d), whatever --steps says
+    # ---- p50 latency of ONE image on ONE replica over --steps images (SURVEY 8d)
     sinks_off()
-    P50_STEPS, P50_WARM = max(200, args.steps), 20
+    P50_STEPS, P50_WARM = args.steps, 20
 
     def step_one(i):
         k = i % NIMG
@@ -633,6 +642,10 @@ def main():
                                 "logical_cpus": os.cpu_count(), "thread_count_proxy_s": tried,
                                 "sample": f"1 full image (1000 ROIs), {dt:.1f} s; dense layers PyTorch-CPU fp32, ROI/decode C restatement, "
                                           f"NMS {'literal nms.c' if use_lit else 'nms.c restatement'}"}
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a, np.float32))
     if rank == 0:
         print(json.dumps(line))
     if world > 1:

@@ -34,6 +34,28 @@ def rel_err(a, b):
     return float(np.max(np.abs(a - b)) / max(np.max(np.abs(b)), 1e-30))
 
 
+_LITERAL = {}
+
+
+def literal_golden(key):
+    """an array stored by tests/golden/make_golden.py from the reference's own nms.c (nms_literal_golden.npz)"""
+    import numpy as np
+    if not _LITERAL:
+        _LITERAL.update(np.load(os.path.join(ROOT, "tests", "golden", "nms_literal_golden.npz")))
+    return _LITERAL[key]
+
+
+def literal_nms_rows(key, scored_boxes, thr):
+    """the rows the reference's own nms.c keeps from `scored_boxes` at `thr`, in its emission order, as stored under `key`;
+    fails when the seeded input is no longer the one the golden was made from"""
+    import hashlib
+    import numpy as np
+    sb = np.ascontiguousarray(scored_boxes, np.float32).reshape(-1, 5)
+    assert hashlib.sha1(sb.tobytes()).hexdigest() == str(literal_golden(key + "_sha1")), f"{key}: input differs from the golden's"
+    assert np.float32(thr) == literal_golden(key + "_thr"), key
+    return sb[literal_golden(key + "_keep")]
+
+
 def record_parity(name, **values):
     """append one JSON line of measured parity figures to $MPN_PARITY_LOG (the GPU run scripts set it; the numbers end up
     under profiles/): the bars are asserted by the tests, the log keeps HOW FAR inside them a run was"""

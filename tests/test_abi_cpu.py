@@ -11,6 +11,7 @@ import multipathnet_b200 as mpn
 from multipathnet_b200 import _lib, models, workloads as wl
 from multipathnet_b200.image_detect import ImageDetect, _image_scale
 from multipathnet_b200.modules import ImageTransformer
+from conftest import literal_golden, literal_nms_rows, rel_err
 
 
 def _header_functions():
@@ -144,9 +145,12 @@ def test_cfg1_alexnet_cpu_plumbing(oracle_built):
     assert bboxes.min() >= 1 and bboxes[:, 0::2].max() <= 224
     ts = G.trunk_forward(spec, img)
     assert tuple(ts[9].shape) == (1, 256, 13, 13)                 # conv5 of CaffeNet at 224 px
+    stored = literal_golden("cfg1_sb")                            # this forward's rows as the golden run computed them
     for j, k in enumerate(keeps, start=1):                        # keep lists = the literal nms.c on the same rows
         sb = np.concatenate([bboxes[:, 4 * j:4 * j + 4], scores[:, j:j + 1]], 1).astype(np.float32)
-        assert np.array_equal(sb[k], O.ref_nms_rows(sb, 0.3))
+        assert rel_err(sb[:, :4], stored[j - 1, :, :4]) < 1e-5 and rel_err(sb[:, 4], stored[j - 1, :, 4]) < 1e-4
+        assert np.array_equal(k, O.nms(sb, 0.3))
+        assert np.array_equal(stored[j - 1][O.nms(stored[j - 1], 0.3)], literal_nms_rows(f"cfg1_class{j}", stored[j - 1], 0.3))
     # the B200 path refuses this configuration loudly (grouped conv + LRN are CPU-plumbing only)
     with pytest.raises(mpn.MpnError):
         mpn.Model.build_desc(spec)

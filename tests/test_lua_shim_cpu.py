@@ -2,6 +2,7 @@
 here): every `C.mpn_*` call names a function the header declares and passes as many arguments as its prototype has,
 every struct type handed to ffi.new exists in the cdef block, and block keywords balance."""
 import glob
+import json
 import os
 import re
 
@@ -125,9 +126,8 @@ def test_image_detect_keeps_the_reference_contract():
     assert "torch.class('fbcoco.ImageDetect')" in raw
     got = _methods(shim)
     assert got == IMAGE_DETECT_API, got
-    ref_path = "/root/reference/ImageDetect.lua"
-    if os.path.exists(ref_path):                                         # the table above IS the reference's (checked where it is present)
-        assert _methods(_strip_lua(open(ref_path).read())) == IMAGE_DETECT_API
+    with open(os.path.join(ROOT, "tests", "golden", "image_detect_api.json")) as f:    # the reference's own table (make_golden.py)
+        assert json.load(f) == IMAGE_DETECT_API
     # the constructor keeps the nn module (Tester_FRCNN.lua:37-49 calls module:apply / module:forward / module.output on it)
     assert re.search(r"self\.model\s*=\s*model\b", shim) and "model_desc.create(" in shim
     # no C handle in a serialisable field: the cache is a weak-keyed table, dropped by clearState

@@ -1,5 +1,5 @@
-"""GPU parity: batched NMS / nms_dense / bbox_vote through the C ABI vs the literal reference nms.c
-(oracle/_ref, when built) and its C restatement. Criterion: BIT-EXACT keep indices / rows."""
+"""GPU parity: batched NMS / nms_dense / bbox_vote through the C ABI vs the literal reference nms.c (its outputs on the
+same seeded inputs, stored by tests/golden/make_golden.py) and its C restatement. Criterion: BIT-EXACT keep indices / rows."""
 import os
 
 import numpy as np
@@ -7,15 +7,15 @@ import pytest
 
 from multipathnet_b200 import workloads as wl
 from oracle import ref as O
+from conftest import literal_golden, literal_nms_rows
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
-def _expect_rows(sb, thr):
+def _expect_rows(key, sb, thr):
     rows = O.nms(sb, thr)
-    if O.ref_available():                       # the literal reference travels to the GPU box as a prebuilt .so
-        assert np.array_equal(sb[rows], O.ref_nms_rows(sb, thr))
+    assert np.array_equal(sb[rows], literal_nms_rows(key, sb, thr))
     return rows
 
 
@@ -23,28 +23,28 @@ def _expect_rows(sb, thr):
 def test_nms_distinct_scores_bit_exact(ctx, n):
     sb = wl.nms_sweep_boxes(n, 1, 1000 + n)[0]
     keep = ctx.nms(sb, 0.3)
-    assert np.array_equal(keep, _expect_rows(sb, 0.3))
+    assert np.array_equal(keep, _expect_rows(f"gpu_distinct_{n}", sb, 0.3))
 
 
 @pytest.mark.parametrize("seed", range(6))
 def test_nms_tied_scores_follow_reference_permutation(ctx, seed):
     """ties: nms.c's selection order is an artefact of its pointer swaps; the exact-emulation kernel must match"""
     sb = wl.nms_sweep_boxes(300 + 97 * seed, 1, 2000 + seed, ties=True)[0]
-    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows(sb, 0.3))
+    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows(f"gpu_ties_{seed}", sb, 0.3))
 
 
 def test_nms_all_equal_scores_and_duplicates(ctx):
     sb = wl.nms_sweep_boxes(257, 1, 5)[0]
     sb[:, 4] = 0.5
-    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows(sb, 0.3))
+    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows("gpu_all_equal", sb, 0.3))
     dup = np.repeat(wl.nms_sweep_boxes(40, 1, 6)[0], 3, axis=0)       # identical boxes AND scores
-    assert np.array_equal(ctx.nms(dup, 0.3), _expect_rows(dup, 0.3))
+    assert np.array_equal(ctx.nms(dup, 0.3), _expect_rows("gpu_duplicates", dup, 0.3))
 
 
 @pytest.mark.parametrize("thr", [0.0, 0.1, 0.3, 0.5, 0.7, 0.99, 1.0])
 def test_nms_thresholds(ctx, thr):
     sb = wl.nms_sweep_boxes(700, 1, 31)[0]
-    assert np.array_equal(ctx.nms(sb, thr), _expect_rows(sb, thr))
+    assert np.array_equal(ctx.nms(sb, thr), _expect_rows(f"gpu_thr_{thr}", sb, thr))
 
 
 def test_nms_empty_and_degenerate_boxes(ctx):
@@ -52,7 +52,7 @@ def test_nms_empty_and_degenerate_boxes(ctx):
     sb = wl.nms_sweep_boxes(200, 1, 8)[0]
     sb[::7, 2] = sb[::7, 0] - 5            # inverted boxes: w<=0 => overlap 0 (nms.c:40)
     sb[::11, :4] = 0
-    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows(sb, 0.3))
+    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows("gpu_degenerate", sb, 0.3))
 
 
 def test_nms_batched_ragged_segments(ctx):
@@ -64,8 +64,8 @@ def test_nms_batched_ragged_segments(ctx):
     sb = np.concatenate(segs, 0)
     offs = np.concatenate([[0], np.cumsum(sizes)])
     keeps = ctx.nms_batched(sb, offs, 0.3)
-    for s, k in zip(segs, keeps):
-        assert np.array_equal(k, _expect_rows(s, 0.3))
+    for i, (s, k) in enumerate(zip(segs, keeps)):
+        assert np.array_equal(k, _expect_rows(f"gpu_ragged_{i}", s, 0.3))
 
 
 def test_nms_80_classes_of_1000(ctx):
@@ -112,8 +112,8 @@ def test_bbox_vote_bit_exact(ctx):
     rows = sb[ctx.nms(sb, 0.3)]
     got = ctx.bbox_vote(rows, sb, 0.5)
     assert np.array_equal(got, O.bbox_vote(rows, sb, 0.5))
-    if O.ref_available():
-        assert np.array_equal(got, O.ref_bbox_vote(rows, sb, 0.5))
+    assert np.array_equal(rows, literal_nms_rows("gpu_vote", sb, 0.3))
+    assert np.array_equal(got, literal_golden("gpu_vote_out"))
 
 
 def test_nms_sweep_50k_single_class(ctx):
@@ -133,9 +133,9 @@ def test_nms_sweep_10k_x_80(ctx):
 def test_nms_medium_segments_with_ties(ctx, n, seed):
     """1024 < n <= 4096: warp-serial walk with the mask in L2 (2 removed-words per lane); 4097: chunked path"""
     sb = wl.nms_sweep_boxes(n, 1, 3000 + seed, ties=True)[0]
-    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows(sb, 0.3))
+    assert np.array_equal(ctx.nms(sb, 0.3), _expect_rows(f"gpu_medium_ties_{n}", sb, 0.3))
     sb2 = wl.nms_sweep_boxes(n, 1, 3100 + seed)[0]
-    assert np.array_equal(ctx.nms(sb2, 0.3), _expect_rows(sb2, 0.3))
+    assert np.array_equal(ctx.nms(sb2, 0.3), _expect_rows(f"gpu_medium_{n}", sb2, 0.3))
 
 
 def test_nms_duplicate_rows_many_classes(ctx):

@@ -1,11 +1,12 @@
 """CPU suite, part 1: pin the oracle against everything the reference's own tests hold for this
-path (SURVEY 8c) and against the literal nms.c compiled into oracle/_ref."""
+path (SURVEY 8c) and against what the literal nms.c returned on the same inputs (tests/golden/make_golden.py)."""
 import os
 
 import numpy as np
 import pytest
 
 from multipathnet_b200 import workloads as wl
+from conftest import literal_golden, literal_nms_rows
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -18,7 +19,7 @@ def test_iou_known_answer(oracle_built):
     gt = np.array([1 / 7, 1 / 3, 1 / 3, 1, 1 / 7], np.float32)
     mine = np.array([O.overlap(x, b) for x in a], np.float32)
     assert np.max(mine - gt) < 5e-3
-    lit = O.ref_boxoverlap(a, b)                      # the literal nms.c:boxoverlap
+    lit = literal_golden("boxoverlap")               # the literal nms.c:boxoverlap
     assert np.array_equal(mine, lit)                  # bit-exact vs the reference's own code
 
 
@@ -52,7 +53,7 @@ def test_nms_restatement_equals_literal_reference(oracle_built, n, seed):
     """orc_nms (index-returning restatement of nms.c:59-108) must reproduce the literal nms.c row for row"""
     O = oracle_built
     sb = wl.nms_sweep_boxes(n, 1, 100 + seed)[0]
-    rows = O.ref_nms_rows(sb, 0.3)
+    rows = literal_nms_rows(f"cpu_distinct_{n}", sb, 0.3)
     keep = O.nms(sb, 0.3)
     assert np.array_equal(sb[keep], rows)
     # distinct scores => the reference keeps rows in descending-score order (SURVEY A.3)
@@ -64,7 +65,7 @@ def test_nms_restatement_ties(oracle_built, seed):
     """tied scores: nms.c's order is an artefact of its swap permutation; the restatement must follow it"""
     O = oracle_built
     sb = wl.nms_sweep_boxes(300, 1, 200 + seed, ties=True)[0]
-    assert np.array_equal(sb[O.nms(sb, 0.3)], O.ref_nms_rows(sb, 0.3))
+    assert np.array_equal(sb[O.nms(sb, 0.3)], literal_nms_rows(f"cpu_ties_{seed}", sb, 0.3))
 
 
 def test_nms_thresholds_and_empty(oracle_built):
@@ -72,14 +73,14 @@ def test_nms_thresholds_and_empty(oracle_built):
     assert len(O.nms(np.zeros((0, 5), np.float32), 0.3)) == 0
     sb = wl.nms_sweep_boxes(200, 1, 9)[0]
     for thr in (0.0, 0.3, 0.5, 0.99, 1.0):
-        assert np.array_equal(sb[O.nms(sb, thr)], O.ref_nms_rows(sb, thr))
+        assert np.array_equal(sb[O.nms(sb, thr)], literal_nms_rows(f"cpu_thr_{thr}", sb, thr))
 
 
 def test_bbox_vote_restatement_equals_literal(oracle_built):
     O = oracle_built
     sb = wl.nms_sweep_boxes(300, 1, 11)[0]
-    rows = O.ref_nms_rows(sb, 0.3)
-    assert np.array_equal(O.bbox_vote(rows, sb, 0.5), O.ref_bbox_vote(rows, sb, 0.5))
+    rows = literal_nms_rows("cpu_vote", sb, 0.3)
+    assert np.array_equal(O.bbox_vote(rows, sb, 0.5), literal_golden("cpu_vote_out"))
 
 
 def test_foveal_regions(oracle_built):
