@@ -198,6 +198,14 @@ void mpn_model_destroy(mpn_model *m);
  * image: 3 x H x W fp32 host (or device with _dev), already transformed+scaled. */
 int mpn_model_trunk(mpn_model *m, const float *image, int32_t H, int32_t W);
 int mpn_model_trunk_dev(mpn_model *m, const float *image_dev, int32_t H, int32_t W);
+/* model:get(1):forward on a batch: images N x 3 x H x W (post-transformer, one size: the caller pads as getImages does,
+ * zeros after the transformer, ImageDetect.lua:44-50), 1 <= N <= MPN_MAX_BATCH. Later mpn_model_heads* / get_pooled /
+ * get_trunk_slot calls see all N images; ROI rows pick their image with column 0 (1-based), and a row naming an image
+ * outside [1, N] fails the call (host entries) or raises the ctx's device flag (_dev entries: the next synchronous call
+ * or mpn_ctx_synchronize fails). N = 1 is exactly mpn_model_trunk(_dev).                                             */
+enum { MPN_MAX_BATCH = 64 };
+int mpn_model_trunk_batch_dev(mpn_model *m, const float *images_dev, int32_t N, int32_t H, int32_t W);
+int mpn_model_trunk_batch(mpn_model *m, const float *images, int32_t N, int32_t H, int32_t W);
 /* ---- getImages on the device (SURVEY 8f-1): ImageDetect.lua:22-52 + modules/ImageTransformer.lua:19-33 ----------
  * fbcoco.ImageTransformer(mean, std, scale, swap) as plain data: out[c] = (im[swap[c]] * scale - mean[c]) / std[c],
  * each step fp32 in that order, `* scale` skipped when scale == 1, `/ std` when has_std == 0 (RossTransformer:
@@ -305,6 +313,22 @@ int mpn_model_detect_nms_dev(mpn_model *m, const float *image_dev, int32_t H, in
                              const float *boxes_dev, int64_t R, float im_scale, float W0, float H0,
                              float score_thresh, float nms_thr, float *scores_dev,
                              float *bboxes_dev, int32_t *keep_idx_dev, int32_t *keep_counts_dev);
+/* mpn_model_detect_nms for N images in one stream-ordered pass: images N x 3 x H x W as mpn_model_trunk_batch. boxes:
+ * R_total x 4, ORIGINAL coordinates of their own image; image i owns rows [img_offsets[i], img_offsets[i+1]) (host, N + 1
+ * entries, img_offsets[0] = 0, every R_i >= 1, R_total <= max_rois). im_scale, W0, H0: host arrays of N. scores R_total x C,
+ * bboxes R_total x 4C (clamped to their own image). keep_idx: image i's (C-1) x R_i block starts at (C-1) * img_offsets[i],
+ * with row indices local to image i; keep_counts N x (C-1). Each image's slice is what mpn_model_detect_nms returns for that
+ * image alone (the trunk's tensor-core plans depend on N, so its last bits may differ; entries of keep_idx past a class's
+ * count are unspecified). With a detection sink set, N records are appended in image order. Any output may be NULL.
+ * _dev: device buffers, stream-ordered; the host form is synchronous.                                                  */
+int mpn_model_detect_nms_batch_dev(mpn_model *m, const float *images_dev, int32_t N, int32_t H, int32_t W,
+                                   const float *boxes_dev, const int64_t *img_offsets, const float *im_scale,
+                                   const float *W0, const float *H0, float score_thresh, float nms_thr,
+                                   float *scores_dev, float *bboxes_dev, int32_t *keep_idx_dev, int32_t *keep_counts_dev);
+int mpn_model_detect_nms_batch(mpn_model *m, const float *images, int32_t N, int32_t H, int32_t W,
+                               const float *boxes, const int64_t *img_offsets, const float *im_scale,
+                               const float *W0, const float *H0, float score_thresh, float nms_thr,
+                               float *scores, float *bboxes, int32_t *keep_idx, int32_t *keep_counts);
 
 /* ---- the detect tail after the network for a RANGE of classes (BASELINE configs[4], "NMS + BBoxNorm sweep": classes
  * shard across GPUs): nn.BBoxNorm (modules/BBoxNorm.lua:18-32; mean4 / std4 NULL = none) + utils.convertFrom per class
@@ -368,7 +392,7 @@ int mpn_dist_nccl_version(mpn_ctx *ctx, int32_t *version);
  * out may be NULL to query *R_total / *bins / *Ctot only. Host buffer, synchronous.                                 */
 int mpn_model_get_pooled(mpn_model *m, int32_t tower, int64_t r0, int64_t n, float *out, int64_t capacity,
                          int64_t *R_total, int32_t *bins, int32_t *Ctot);
-/* introspection for tests/profiling: copy a trunk slot to host as N x C x H x W fp32 */
+/* introspection for tests/profiling: copy a trunk slot to host as N x C x H x W fp32 (N = images of the last trunk call) */
 int mpn_model_get_trunk_slot(mpn_model *m, int32_t slot, float *out_nchw, int64_t capacity,
                              int32_t *C, int32_t *H, int32_t *W);
 /* select conv/GEMM implementation: 0 = tcgen05 tensor-core path (default, product),

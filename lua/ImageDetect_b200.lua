@@ -88,7 +88,7 @@ local function transform_struct(t)   -- fbcoco.ImageTransformer fields (ImageTra
 end
 ImageDetect._transform_struct = transform_struct
 
--- ImageDetect.lua:91-135. input = {images 1 x 3 x H x W, rois R x 5}, CudaTensors (what detect / the Tester hand over).
+-- ImageDetect.lua:91-135. input = {images N x 3 x H x W, rois R x 5}, CudaTensors (what detect / the Tester hand over).
 -- The trunk runs once, the heads on ALL rois in one pass: the reference chunks by `bs` only to bound memory, and its own
 -- self-test (:126-133) demands chunked == unchunked exactly, which the library guarantees (row-chunk invariance), so
 -- `bs` is accepted and ignored. Device pointers go straight through: no host round trip.
@@ -106,8 +106,13 @@ function ImageDetect:memoryEfficientForward(model, input, bs, recompute_features
    self.output[2]:resize(R, nc * 4)
    local ctx = mpn.ctx()
    if recompute_features then
-      assert(images:size(1) >= 1 and images:size(2) == 3)     -- min_images copies (:143-146) are replicas: image 1 is the image
-      mpn.check(ctx, C.mpn_model_trunk_dev(h.handle, mpn.fptr(images), images:size(3), images:size(4)), 'mpn_model_trunk_dev')
+      assert(images:size(1) >= 1 and images:size(2) == 3)
+      if images:size(1) == 1 then
+         mpn.check(ctx, C.mpn_model_trunk_dev(h.handle, mpn.fptr(images), images:size(3), images:size(4)), 'mpn_model_trunk_dev')
+      else   -- a padded batch: every image goes through the trunk, ROI rows pick theirs with column 1 (1-based)
+         mpn.check(ctx, C.mpn_model_trunk_batch_dev(h.handle, mpn.fptr(images), images:size(1), images:size(3), images:size(4)),
+                   'mpn_model_trunk_batch_dev')
+      end
    end
    mpn.check(ctx, C.mpn_model_heads_dev(h.handle, mpn.fptr(rois), R, mpn.fptr(self.output[1]), mpn.fptr(self.output[2])), 'mpn_model_heads_dev')
    return self.output

@@ -12,7 +12,7 @@ build image — see INTEGRATION.md for the LuaJIT-FFI shim in lua/) of:
 All compute happens in libmpn_b200.so (hand-written CUDA); nothing here falls back to CPU.
 """
 from ._lib import (Context, Model, ModelSpec, MpnError, load_library, LIB_PATH,  # noqa: F401
-                   MPN_MAX_DET, MPN_REC_FLOATS, MPN_DIST_ID_BYTES)
+                   MPN_MAX_DET, MPN_REC_FLOATS, MPN_DIST_ID_BYTES, MPN_MAX_BATCH)
 from . import models, modules, t7, utils, workloads  # noqa: F401
 from .image_detect import ImageDetect  # noqa: F401
 from .tester import Tester  # noqa: F401

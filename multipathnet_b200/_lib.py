@@ -19,7 +19,7 @@ LIB_PATH = os.path.join(_HERE, "libmpn_b200.so")
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "mpn_abi.h")
 
 MPN_LAYER_CONV, MPN_LAYER_MAXPOOL, MPN_LAYER_AVGPOOL, MPN_LAYER_FLATTEN = 1, 2, 3, 4
-MPN_MAX_DET, MPN_REC_FLOATS, MPN_DIST_ID_BYTES = 128, 769, 128      # include/mpn_abi.h
+MPN_MAX_DET, MPN_REC_FLOATS, MPN_DIST_ID_BYTES, MPN_MAX_BATCH = 128, 769, 128, 64      # include/mpn_abi.h
 MPN_LAYER_LRN = 5       # CaffeNet local response norm: CPU-oracle plumbing config only (BASELINE configs[0]), not on the B200 path
 
 
@@ -127,6 +127,12 @@ SIGNATURES = {
     "mpn_model_destroy": (None, [_vp]),
     "mpn_model_trunk": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32]),
     "mpn_model_trunk_dev": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32]),
+    "mpn_model_trunk_batch": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32]),
+    "mpn_model_trunk_batch_dev": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32]),
+    "mpn_model_detect_nms_batch": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, _vp, _i64p, _vp, _vp, _vp, C.c_float, C.c_float,
+                                             _vp, _vp, _vp, _vp]),
+    "mpn_model_detect_nms_batch_dev": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, _vp, _i64p, _vp, _vp, _vp, C.c_float,
+                                                 C.c_float, _vp, _vp, _vp, _vp]),
     "mpn_model_heads": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp]),
     "mpn_model_heads_dev": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp]),
     "mpn_model_detect": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, _vp, C.c_int64, C.c_float, C.c_int32, _vp, _vp]),
@@ -583,6 +589,8 @@ class Model:
                   "mpn_model_create")
         self.h = h
         self.C = spec.num_classes
+        self.max_rois = int(max_rois)
+        self._trunk_n = 1                  # images of the last trunk forward (the leading size of trunk_slot)
         import weakref
         ctx._models.append(weakref.ref(self))
 
@@ -624,7 +632,16 @@ class Model:
     def trunk(self, image_chw):
         im = _f32(image_chw)
         assert im.ndim == 3 and im.shape[0] == 3
+        self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_trunk(self.h, _ptr(im), im.shape[1], im.shape[2]), "mpn_model_trunk")
+
+    def trunk_batch(self, images_nchw):
+        """model:get(1):forward on N x 3 x H x W images of one (padded) size; ROI rows then pick their image by column 0"""
+        im = _f32(images_nchw)
+        if im.ndim != 4 or im.shape[1] != 3 or im.shape[0] < 1 or im.shape[0] > MPN_MAX_BATCH:
+            raise ValueError(f"trunk_batch expects N x 3 x H x W images with 1 <= N <= {MPN_MAX_BATCH}")
+        self._trunk_n = im.shape[0]
+        self.ctx.check(self.ctx.lib.mpn_model_trunk_batch(self.h, _ptr(im), im.shape[0], im.shape[2], im.shape[3]), "mpn_model_trunk_batch")
 
     def trunk_image(self, raw_image_chw, kind: str, scale: float = 600, max_size: float = 1000):
         """getImages + trunk on the device from the RAW image (SURVEY 8f-1) -> (im_scale, h, w)"""
@@ -633,6 +650,7 @@ class Model:
             raise ValueError("ImageTransformer expects a 3 x H x W image")
         h, w, s = C.c_int32(), C.c_int32(), C.c_double()
         tf = CImageTransform.of(kind)
+        self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_trunk_image(self.h, _ptr(im), im.shape[1], im.shape[2], C.addressof(tf), float(scale),
                                                           float(max_size), C.byref(s), C.byref(h), C.byref(w)), "mpn_model_trunk_image")
         return float(s.value), h.value, w.value
@@ -645,9 +663,13 @@ class Model:
         self.ctx.check(self.ctx.lib.mpn_model_heads(self.h, _ptr(r), n, _ptr(cls), _ptr(bbox)), "mpn_model_heads")
         return cls, bbox
 
-    def forward(self, image_chw, rois):
-        """model:forward{images, rois} (eval mode)."""
-        self.trunk(image_chw)
+    def forward(self, images, rois):
+        """model:forward{images, rois} (eval mode): images 3 x H x W, or N x 3 x H x W with ROI rows [n, x1, y1, x2, y2]
+        naming their image by the 1-based n."""
+        if np.ndim(images) == 4:
+            self.trunk_batch(images)
+        else:
+            self.trunk(images)
         return self.heads(rois)
 
     def detect(self, image_chw, boxes, im_scale: float, recompute_features: bool = True):
@@ -657,6 +679,8 @@ class Model:
         scores = np.empty((n, self.C), dtype=np.float32)
         bboxes = np.empty((n, 4 * self.C), dtype=np.float32)
         H, W = (im.shape[1], im.shape[2]) if im is not None else (0, 0)
+        if recompute_features:
+            self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_detect(self.h, _ptr(im), H, W, _ptr(b), n, float(im_scale),
                                                      int(recompute_features), _ptr(scores), _ptr(bboxes)), "mpn_model_detect")
         return scores, bboxes
@@ -669,6 +693,7 @@ class Model:
         bboxes = np.empty((n, 4 * self.C), dtype=np.float32) if want_raw else None
         keep = np.empty((self.C - 1, n), dtype=np.int32)
         counts = np.empty(self.C - 1, dtype=np.int32)
+        self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_detect_nms(
             self.h, _ptr(im), im.shape[1], im.shape[2], _ptr(b), n, float(im_scale), float(W0), float(H0),
             float(score_thresh), float(nms_thr), _ptr(scores), _ptr(bboxes), _ptr(keep), _ptr(counts)), "mpn_model_detect_nms")
@@ -686,6 +711,7 @@ class Model:
         scores = np.empty((n_out, self.C), np.float32); bboxes = np.empty((n_out, 4 * self.C), np.float32)
         keep = np.empty((self.C - 1, n_out), np.int32); counts = np.empty(self.C - 1, np.int32)
         voted = np.empty((self.C - 1, n_out, 5), np.float32) if bbox_voting else None
+        self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_test_one(self.h, _ptr(im), im.shape[1], im.shape[2], _ptr(b), n, float(im_scale), float(W0), float(H0),
                                                        C.byref(o), _ptr(scores), _ptr(bboxes), _ptr(keep), _ptr(counts), _ptr(voted)), "mpn_model_test_one")
         keeps = [keep[j, :counts[j]].copy() for j in range(self.C - 1)]
@@ -700,6 +726,7 @@ class Model:
         out = dict(im=im, b=b, scores=np.empty((n, self.C), dtype=np.float32), bboxes=np.empty((n, 4 * self.C), dtype=np.float32),
                    keep=np.empty((self.C - 1, n), dtype=np.int32), counts=np.empty(self.C - 1, dtype=np.int32))
         t = C.c_int32(-1)
+        self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_detect_nms_submit(
             self.h, _ptr(im), im.shape[1], im.shape[2], _ptr(b), n, float(im_scale), float(W0), float(H0), float(score_thresh),
             float(nms_thr), _ptr(out["scores"]), _ptr(out["bboxes"]), _ptr(out["keep"]), _ptr(out["counts"]), C.byref(t)),
@@ -716,6 +743,7 @@ class Model:
         out = dict(im=im, b=b, scores=np.empty((n, self.C), dtype=np.float32), bboxes=np.empty((n, 4 * self.C), dtype=np.float32),
                    keep=np.empty((self.C - 1, n), dtype=np.int32), counts=np.empty(self.C - 1, dtype=np.int32), tf=CImageTransform.of(kind))
         t = C.c_int32(-1)
+        self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_detect_nms_submit_u8(
             self.h, _ptr(im), im.shape[0], im.shape[1], C.addressof(out["tf"]), float(scale), float(max_size), _ptr(b), n, float(score_thresh),
             float(nms_thr), _ptr(out["scores"]), _ptr(out["bboxes"]), _ptr(out["keep"]), _ptr(out["counts"]), C.byref(t)),
@@ -733,15 +761,70 @@ class Model:
                        score_thresh: float, nms_thr: float, scores_dev=None, bboxes_dev=None, keep_idx_dev=None,
                        keep_counts_dev=None):
         """Fully device-resident, asynchronous (arguments are torch CUDA tensors or raw addresses)."""
+        self._trunk_n = 1
         self.ctx.check(self.ctx.lib.mpn_model_detect_nms_dev(
             self.h, _ptr(image_dev), H, W, _ptr(boxes_dev), R, float(im_scale), float(W0), float(H0), float(score_thresh),
             float(nms_thr), _ptr(scores_dev), _ptr(bboxes_dev), _ptr(keep_idx_dev), _ptr(keep_counts_dev)),
             "mpn_model_detect_nms_dev")
 
+    def _batch_args(self, N: int, R: Sequence[int], im_scales, sizes):
+        """host-side checks of a batch description -> (img_offsets int64 N+1, im_scale, W0, H0 float32 N)"""
+        if not 1 <= N <= MPN_MAX_BATCH:
+            raise ValueError(f"batch size must be in 1..{MPN_MAX_BATCH}, got {N}")
+        R = [int(r) for r in R]
+        if len(R) != N or len(im_scales) != N or len(sizes) != N:
+            raise ValueError(f"{N} images need {N} box arrays, im_scales and (W0, H0) sizes; got {len(R)}, {len(im_scales)}, {len(sizes)}")
+        if min(R) < 1:
+            raise ValueError("every image needs at least one proposal")
+        offs = np.zeros(N + 1, np.int64)
+        offs[1:] = np.cumsum(R)
+        if offs[-1] > self.max_rois:
+            raise ValueError(f"{int(offs[-1])} proposals in the batch exceed max_rois = {self.max_rois}")
+        sz = np.asarray(sizes, np.float32).reshape(N, 2)
+        return offs, np.asarray(im_scales, np.float32).reshape(N), np.ascontiguousarray(sz[:, 0]), np.ascontiguousarray(sz[:, 1])
+
+    def detect_nms_batch(self, images_nchw, boxes_list, im_scales, sizes, score_thresh: float = -1.5, nms_thr: float = 0.3):
+        """detect_nms for N images of one padded size in one pass: boxes_list[i] R_i x 4 in image i's ORIGINAL coordinates,
+        im_scales[i] and sizes[i] = (W0, H0) as getImages gave them. -> one (scores, bboxes, keeps) per image, as detect_nms."""
+        im = _f32(images_nchw)
+        if im.ndim != 4 or im.shape[1] != 3:
+            raise ValueError("detect_nms_batch expects N x 3 x H x W images")
+        N = im.shape[0]
+        boxes = [_f32(b).reshape(-1, 4) for b in boxes_list]
+        offs, sc, w0, h0 = self._batch_args(N, [b.shape[0] for b in boxes], im_scales, sizes)
+        Rt, Cn = int(offs[-1]), self.C
+        b = np.ascontiguousarray(np.concatenate(boxes, 0))
+        scores = np.empty((Rt, Cn), np.float32); bboxes = np.empty((Rt, 4 * Cn), np.float32)
+        keep = np.empty((Cn - 1) * Rt, np.int32); counts = np.empty((N, Cn - 1), np.int32)
+        self._trunk_n = N
+        self.ctx.check(self.ctx.lib.mpn_model_detect_nms_batch(
+            self.h, _ptr(im), N, im.shape[2], im.shape[3], _ptr(b), offs.ctypes.data_as(_i64p), _ptr(sc), _ptr(w0), _ptr(h0),
+            float(score_thresh), float(nms_thr), _ptr(scores), _ptr(bboxes), _ptr(keep), _ptr(counts)), "mpn_model_detect_nms_batch")
+        out = []
+        for i in range(N):
+            r0, r1 = int(offs[i]), int(offs[i + 1])
+            k = keep[(Cn - 1) * r0:(Cn - 1) * r1].reshape(Cn - 1, r1 - r0)
+            out.append((scores[r0:r1], bboxes[r0:r1], [k[j, :counts[i, j]].copy() for j in range(Cn - 1)]))
+        return out
+
+    def detect_nms_batch_dev(self, images_dev, N: int, H: int, W: int, boxes_dev, R_list: Sequence[int], im_scales, sizes,
+                             score_thresh: float, nms_thr: float, scores_dev=None, bboxes_dev=None, keep_idx_dev=None,
+                             keep_counts_dev=None):
+        """detect_nms_batch fully device-resident and asynchronous (arguments are torch CUDA tensors or raw addresses):
+        boxes_dev R_total x 4, image i owning R_list[i] consecutive rows; keep_idx_dev (C-1) * R_total, image i's
+        (C-1) x R_i block at (C-1) * offset_i; keep_counts_dev N x (C-1)."""
+        offs, sc, w0, h0 = self._batch_args(int(N), R_list, im_scales, sizes)
+        self._trunk_n = int(N)
+        self.ctx.check(self.ctx.lib.mpn_model_detect_nms_batch_dev(
+            self.h, _ptr(images_dev), int(N), int(H), int(W), _ptr(boxes_dev), offs.ctypes.data_as(_i64p), _ptr(sc), _ptr(w0),
+            _ptr(h0), float(score_thresh), float(nms_thr), _ptr(scores_dev), _ptr(bboxes_dev), _ptr(keep_idx_dev),
+            _ptr(keep_counts_dev)), "mpn_model_detect_nms_batch_dev")
+
     def trunk_slot(self, slot: int) -> np.ndarray:
+        """trunk slot `slot` of the last trunk forward as N x C x H x W fp32 (N = its images)"""
         c, h, w = C.c_int32(), C.c_int32(), C.c_int32()
         self.ctx.check(self.ctx.lib.mpn_model_get_trunk_slot(self.h, slot, None, 0, C.byref(c), C.byref(h), C.byref(w)), "get_trunk_slot")
-        out = np.empty((1, c.value, h.value, w.value), dtype=np.float32)
+        out = np.empty((self._trunk_n, c.value, h.value, w.value), dtype=np.float32)
         self.ctx.check(self.ctx.lib.mpn_model_get_trunk_slot(self.h, slot, _ptr(out), out.size, C.byref(c), C.byref(h), C.byref(w)),
                        "get_trunk_slot")
         return out

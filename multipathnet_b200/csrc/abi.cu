@@ -58,8 +58,12 @@ int mpn_ovf_copy_async(mpn_ctx *ctx, cudaStream_t stream) {
 }
 int mpn_ovf_test(mpn_ctx *ctx) {
   if (!ctx->ovf_dev || !*ctx->ovf_host) return MPN_OK;
+  const unsigned bits = *ctx->ovf_host;
   *ctx->ovf_host = 0;
   MPN_CUDA(ctx, cudaMemsetAsync(ctx->ovf_dev, 0, sizeof(unsigned), ctx->stream));
+  if (bits & MPN_FLAG_BAD_BATCH)
+    return mpn_fail(ctx, MPN_ERR_ARG, "a ROI row's batch index (column 0, 1-based, ImageDetect.lua:69) lies outside [1, N] for the N "
+                                      "images of the last trunk forward: results of this call are invalid");
   return mpn_fail(ctx, MPN_ERR_STATE, "an activation left fp16's range (|x| > 65504 or NaN) in the fp16-plane path of fc6 / fc7: results of this call are "
                                       "saturated; rerun with mpn_ctx_set_option(ctx, \"fc_w16\", 0) (or MPN_FC_W16=0) for the three-product bf16 path");
 }

@@ -126,9 +126,11 @@ inline cudaError_t mpn_launch_pdl(mpn_ctx *ctx, void (*kern)(KArgs...), dim3 gri
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 
-int mpn_ovf_flag(mpn_ctx *ctx, unsigned **flag_dev);          // the ctx's fp16-overflow flag (allocated on first use)
+// bits of the device flag word: an fp16 activation plane saturated / a ROI row named an image outside [1, N]
+enum { MPN_FLAG_FP16_OVF = 1u, MPN_FLAG_BAD_BATCH = 2u };
+int mpn_ovf_flag(mpn_ctx *ctx, unsigned **flag_dev);          // the ctx's device flag word (allocated on first use)
 // enqueue the copy of the flag to its pinned host word on `stream` (no-op without a flag) / after that stream was
-// synchronised: fail loudly if an fp16 activation plane saturated since the last test, and re-arm the flag
+// synchronised: fail loudly if a flag bit was raised since the last test, and re-arm the flag
 int mpn_ovf_copy_async(mpn_ctx *ctx, cudaStream_t stream);
 int mpn_ovf_test(mpn_ctx *ctx);
 int mpn_scratch(mpn_ctx *ctx, size_t bytes, void **out);    // slot 1
@@ -194,3 +196,16 @@ struct DTensor {
   int64_t N = 0, H = 0, W = 0, C = 0, ld = 0;
   int64_t pixels() const { return N * H * W; }
 };
+
+// The images of a batched detect tail (mpn_model_detect_nms_batch*), passed by value to its kernels: image i owns proposal
+// rows [off[i], off[i + 1]) and has its own im_scale and original size.
+struct MpnBatch {
+  int n;
+  int off[MPN_MAX_BATCH + 1];
+  float scale[MPN_MAX_BATCH], W0[MPN_MAX_BATCH], H0[MPN_MAX_BATCH];
+};
+__device__ __forceinline__ int mpn_batch_image(const MpnBatch &b, int64_t row) {   // the image owning proposal row `row`
+  int i = 0;
+  while (i + 1 < b.n && row >= b.off[i + 1]) ++i;
+  return i;
+}

@@ -133,15 +133,25 @@ detect_tail_kernel(const float *__restrict__ logits, int64_t R, int C, int K, in
   else bbox_decode_body((int64_t)(blockIdx.x - nb_sm) * 256 + threadIdx.x, deltas, boxes, R, C, do_clamp, W0, H0, bboxes, has_norm, mean, stdv);
 }
 
+// batched detect tail: the same blocks, every decoded row clamped to its own image's W0 x H0 (Tester_FRCNN.lua:75-78)
+__global__ void __launch_bounds__(256)
+detect_tail_batch_kernel(const float *__restrict__ logits, int64_t R, int C, int K, int do_softmax, float *__restrict__ scores,
+                         int nb_sm, const float *__restrict__ deltas, const float *__restrict__ boxes, const MpnBatch b,
+                         float *__restrict__ bboxes, int has_norm, float4 mean, float4 stdv) {
+  MPN_PDL_SYNC();
+  if ((int)blockIdx.x < nb_sm) { softmax_mean_body((int64_t)blockIdx.x * 256 + threadIdx.x, logits, R, C, K, do_softmax, scores); return; }
+  const int64_t idx = (int64_t)(blockIdx.x - nb_sm) * 256 + threadIdx.x;
+  const int img = mpn_batch_image(b, idx / C);
+  bbox_decode_body(idx, deltas, boxes, R, C, 1, b.W0[img], b.H0[img], bboxes, has_norm, mean, stdv);
+}
+
 // ---- Tester_FRCNN.lua:106-116: per foreground class j gather rows with score > thresh ----
 // into seg j-1: sb[seg][k] = [bbox(:,4j..4j+3), score(:,j)], order preserved (stable), plus
 // src_idx[seg][k] = original ROI row and counts[seg]. One block per class.
-__global__ void __launch_bounds__(256)
-gather_scored_kernel(const float *__restrict__ scores, const float *__restrict__ bboxes, int R, int C,
-                     float thresh, float *__restrict__ sb, int32_t *__restrict__ src_idx,
-                     int32_t *__restrict__ counts) {
-  MPN_PDL_SYNC();
-  const int seg = blockIdx.x, j = seg + 1;
+// body for one (image, class) segment: rows [0, R) of scores / bboxes, class j, outputs at sb / src_idx (capacity >= R)
+__device__ __forceinline__ void gather_scored_body(const float *__restrict__ scores, const float *__restrict__ bboxes, int R, int C,
+                                                   int j, float thresh, float *__restrict__ sb, int32_t *__restrict__ src_idx,
+                                                   int32_t *__restrict__ count) {
   __shared__ int s_wtot[8];
   __shared__ int s_total;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -163,14 +173,32 @@ gather_scored_kernel(const float *__restrict__ scores, const float *__restrict__
     if (flag) {
       int k = base_out + s_wtot[wid] + pre;
       float4 b = reinterpret_cast<const float4 *>(bboxes)[(size_t)r * C + j];
-      float *o = sb + ((size_t)seg * R + k) * 5;
+      float *o = sb + (size_t)k * 5;
       o[0] = b.x; o[1] = b.y; o[2] = b.z; o[3] = b.w; o[4] = s;
-      src_idx[(size_t)seg * R + k] = r;
+      src_idx[k] = r;
     }
     base_out += s_total;
     __syncthreads();
   }
-  if (threadIdx.x == 0) counts[seg] = base_out;
+  if (threadIdx.x == 0) *count = base_out;
+}
+__global__ void __launch_bounds__(256)
+gather_scored_kernel(const float *__restrict__ scores, const float *__restrict__ bboxes, int R, int C,
+                     float thresh, float *__restrict__ sb, int32_t *__restrict__ src_idx,
+                     int32_t *__restrict__ counts) {
+  MPN_PDL_SYNC();
+  const int seg = blockIdx.x;
+  gather_scored_body(scores, bboxes, R, C, seg + 1, thresh, sb + (size_t)seg * R * 5, src_idx + (size_t)seg * R, counts + seg);
+}
+// batched form: grid (C - 1, N); segment (image i, class j) = i * (C - 1) + j - 1 at capacity cap, row indices local to image i
+__global__ void __launch_bounds__(256)
+gather_scored_batch_kernel(const float *__restrict__ scores, const float *__restrict__ bboxes, int C, float thresh, const MpnBatch b,
+                           int cap, float *__restrict__ sb, int32_t *__restrict__ src_idx, int32_t *__restrict__ counts) {
+  MPN_PDL_SYNC();
+  const int img = blockIdx.y, r0 = b.off[img];
+  const size_t seg = (size_t)img * (C - 1) + blockIdx.x;
+  gather_scored_body(scores + (size_t)r0 * C, bboxes + (size_t)r0 * 4 * C, b.off[img + 1] - r0, C, blockIdx.x + 1, thresh,
+                     sb + seg * cap * 5, src_idx + seg * cap, counts + seg);
 }
 
 // ---- max-pool k x k / stride / pad on split-bf16 NHWC planes, 8 channels per thread ------
@@ -295,6 +323,22 @@ __global__ void project_rois_kernel(const float *__restrict__ boxes, int64_t R, 
   float4 b = reinterpret_cast<const float4 *>(boxes)[i];
   float *o = rois + i * 5;
   o[0] = 1.0f;
+  o[1] = __fadd_rn(__fmul_rn(__fsub_rn(b.x, 1.0f), im_scale), 1.0f);
+  o[2] = __fadd_rn(__fmul_rn(__fsub_rn(b.y, 1.0f), im_scale), 1.0f);
+  o[3] = __fadd_rn(__fmul_rn(__fsub_rn(b.z, 1.0f), im_scale), 1.0f);
+  o[4] = __fadd_rn(__fmul_rn(__fsub_rn(b.w, 1.0f), im_scale), 1.0f);
+}
+
+// batched form: row i belongs to image b(i), projected with that image's im_scale, batch index b(i) + 1
+__global__ void project_rois_batch_kernel(const float *__restrict__ boxes, int64_t R, const MpnBatch bt, float *__restrict__ rois) {
+  MPN_PDL_SYNC();
+  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= R) return;
+  const int img = mpn_batch_image(bt, i);
+  const float im_scale = bt.scale[img];
+  float4 b = reinterpret_cast<const float4 *>(boxes)[i];
+  float *o = rois + i * 5;
+  o[0] = (float)(img + 1);
   o[1] = __fadd_rn(__fmul_rn(__fsub_rn(b.x, 1.0f), im_scale), 1.0f);
   o[2] = __fadd_rn(__fmul_rn(__fsub_rn(b.y, 1.0f), im_scale), 1.0f);
   o[3] = __fadd_rn(__fmul_rn(__fsub_rn(b.z, 1.0f), im_scale), 1.0f);
@@ -499,6 +543,34 @@ int mpn_project_rois_launch(mpn_ctx *ctx, const float *boxes_dev, int64_t R, flo
   MpnProfScope prof_scope__(ctx, MPN_CAT_ELTWISE);
   if (R <= 0) return MPN_OK;
   MPN_CUDA(ctx, mpn_launch_pdl(ctx, project_rois_kernel, dim3(nblk(R, 128)), dim3(128), 0, boxes_dev, R, im_scale, rois_dev));
+  MPN_LAUNCHED(ctx);
+  return MPN_OK;
+}
+int mpn_project_rois_batch_launch(mpn_ctx *ctx, const float *boxes_dev, int64_t R, const MpnBatch &b, float *rois_dev) {
+  MpnProfScope prof_scope__(ctx, MPN_CAT_ELTWISE);
+  if (R <= 0) return MPN_OK;
+  MPN_CUDA(ctx, mpn_launch_pdl(ctx, project_rois_batch_kernel, dim3(nblk(R, 128)), dim3(128), 0, boxes_dev, R, b, rois_dev));
+  MPN_LAUNCHED(ctx);
+  return MPN_OK;
+}
+int mpn_detect_tail_batch_launch(mpn_ctx *ctx, const float *logits_dev, int64_t R, int C, int K, int do_softmax, float *scores_dev,
+                                 const float *deltas_dev, const float *boxes_dev, const MpnBatch &b, float *bboxes_dev, int has_norm,
+                                 const float *mean4, const float *std4) {
+  MpnProfScope prof_scope__(ctx, MPN_CAT_ELTWISE);
+  if (R <= 0) return MPN_OK;
+  const int nb_sm = (int)nblk(R * 32, 256), nb_dec = (int)nblk(R * C, 256);
+  MPN_CUDA(ctx, mpn_launch_pdl(ctx, detect_tail_batch_kernel, dim3(nb_sm + nb_dec), dim3(256), 0,
+      logits_dev, R, C, K, do_softmax, scores_dev, nb_sm, deltas_dev, boxes_dev, b, bboxes_dev, has_norm,
+      make_float4(mean4[0], mean4[1], mean4[2], mean4[3]), make_float4(std4[0], std4[1], std4[2], std4[3])));
+  MPN_LAUNCHED(ctx);
+  return MPN_OK;
+}
+int mpn_gather_scored_batch_launch(mpn_ctx *ctx, const float *scores_dev, const float *bboxes_dev, int C, float thresh, const MpnBatch &b,
+                                   int cap, float *sb_dev, int32_t *src_idx_dev, int32_t *counts_dev) {
+  MpnProfScope prof_scope__(ctx, MPN_CAT_ELTWISE);
+  if (C <= 1 || b.n <= 0) return MPN_OK;
+  MPN_CUDA(ctx, mpn_launch_pdl(ctx, gather_scored_batch_kernel, dim3(C - 1, b.n), dim3(256), 0, scores_dev, bboxes_dev, C, thresh, b, cap,
+                               sb_dev, src_idx_dev, counts_dev));
   MPN_LAUNCHED(ctx);
   return MPN_OK;
 }

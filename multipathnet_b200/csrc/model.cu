@@ -21,6 +21,10 @@ int mpn_avgpool_launch(mpn_ctx *, const DTensor &, DTensor &);
 int mpn_weight_permute_split_launch(mpn_ctx *, const float *, int64_t, int, int, int, __nv_bfloat16 *, __nv_bfloat16 *);
 int mpn_nhwc_split_to_nchw_launch(mpn_ctx *, const DTensor &, float *);
 int mpn_project_rois_launch(mpn_ctx *, const float *, int64_t, float, float *);
+int mpn_project_rois_batch_launch(mpn_ctx *, const float *, int64_t, const MpnBatch &, float *);
+int mpn_detect_tail_batch_launch(mpn_ctx *, const float *, int64_t, int, int, int, float *, const float *, const float *, const MpnBatch &,
+                                 float *, int, const float *, const float *);
+int mpn_gather_scored_batch_launch(mpn_ctx *, const float *, const float *, int, float, const MpnBatch &, int, float *, int32_t *, int32_t *);
 int mpn_get_images_launch(mpn_ctx *, const float *, int32_t, int32_t, const mpn_image_transform *, int32_t, int32_t, float *);
 int mpn_get_images_size_impl(int32_t, int32_t, double, double, int32_t *, int32_t *, double *);
 int mpn_get_images_u8_launch(mpn_ctx *, const uint8_t *, int32_t, int32_t, const mpn_image_transform *, int32_t, int32_t, float *);
@@ -101,7 +105,7 @@ struct mpn_model {
   int conv_impl = 0;
 
   // ---- trunk state
-  int tH = 0, tW = 0; bool trunk_valid = false;
+  int tN = 0, tH = 0, tW = 0; bool trunk_valid = false;   // images, height, width the trunk is planned for
   std::vector<LayerExec> trunk_exec;
   std::map<int, DTensor> trunk_slots; std::map<int, std::unique_ptr<SplitBuf>> trunk_bufs;
   DevBuf image_dev, raw_image_dev;
@@ -245,11 +249,11 @@ int run_conv(mpn_model *m, LayerExec &e) {
 }
 
 // ------------------------------------------------------------------ trunk planning
-int plan_trunk(mpn_model *m, int H, int W) {
+int plan_trunk(mpn_model *m, int N, int H, int W) {
   mpn_ctx *ctx = m->ctx;
   m->trunk_exec.clear(); m->trunk_slots.clear();
   m->trunk_flops = 0;
-  DTensor img; img.N = 1; img.H = H; img.W = W; img.C = 3; img.ld = 3;   // slot 0: NCHW fp32 image (special)
+  DTensor img; img.N = N; img.H = H; img.W = W; img.C = 3; img.ld = 3;   // slot 0: NCHW fp32 image (special)
   m->trunk_slots[0] = img;
   for (const mpn_layer &L : m->trunk_layers) {
     MPN_CHECK_ARG(ctx, m->trunk_slots.count(L.in_slot), "trunk layer reads an undefined slot");
@@ -334,7 +338,7 @@ int plan_trunk(mpn_model *m, int H, int W) {
         MPN_TRY(P.lv[k]->ensure(ctx, sizeof(float) * (size_t)(f.N * f.H * f.W * f.C) + 256));
       }
     }
-  m->tH = H; m->tW = W; m->trunk_valid = false; m->heads_planned = false;
+  m->tN = N; m->tH = H; m->tW = W; m->trunk_valid = false; m->heads_planned = false;
   return MPN_OK;
 }
 
@@ -355,7 +359,7 @@ int run_trunk(mpn_model *m, const float *image_dev) {
     if (L.kind == MPN_LAYER_CONV) {
       if (e.is_direct) {
         const float *bias = L.bias >= 0 ? (const float *)m->weights[L.bias]->f32.p : nullptr;
-        MPN_TRY(conv_direct_nchw_launch(ctx, image_dev, 1, L.cin, (int)e.in.H, (int)e.in.W,
+        MPN_TRY(conv_direct_nchw_launch(ctx, image_dev, m->tN, L.cin, (int)e.in.H, (int)e.in.W,
                                         (const float *)m->weights[L.weight]->f32.p, bias, L.cout, L.kh, L.kw, L.stride,
                                         L.pad, L.relu, e.out,
                                         m->w_host_small[L.weight].empty() ? nullptr : m->w_host_small[L.weight].data(),
@@ -421,7 +425,8 @@ int plan_heads(mpn_model *m, int64_t R) {
       MPN_CHECK_ARG(ctx, m->jobs.n < MAX_ROI_JOBS, "too many (tower, level) ROI jobs");
       const DTensor &f = m->trunk_slots[T.level_slot[l]];
       RoiJob &j = m->jobs.j[m->jobs.n++];
-      j.H = (int)f.H; j.W = (int)f.W; j.C = (int)f.C; j.scale = T.level_scale[l];
+      j.H = (int)f.H; j.W = (int)f.W; j.C = (int)f.C; j.nimg = (int)f.N; j.scale = T.level_scale[l];
+      MPN_TRY(mpn_ovf_flag(ctx, &j.flag));
       j.region = T.region; j.out_hi = X.pooled.hi; j.out_lo = X.pooled.lo; j.out_ld = X.ctot; j.out_ch_off = ch_off;
       j.normalize = T.normalize; j.out_fmt = 0; j.ovf = nullptr; j.tower = (int)t;
       const mpn_model::Pyramid &P = m->pyramids[T.level_slot[l]];
@@ -656,8 +661,8 @@ int run_heads(mpn_model *m, const float *rois_dev, int64_t R, bool apply_bbox_no
   return MPN_OK;
 }
 
-int ensure_trunk(mpn_model *m, int H, int W) {
-  if (m->trunk_exec.empty() || m->tH != H || m->tW != W) MPN_TRY(plan_trunk(m, H, W));
+int ensure_trunk(mpn_model *m, int N, int H, int W) {
+  if (m->trunk_exec.empty() || m->tN != N || m->tH != H || m->tW != W) MPN_TRY(plan_trunk(m, N, H, W));
   return MPN_OK;
 }
 int ensure_heads(mpn_model *m, int64_t R) {
@@ -729,13 +734,31 @@ int mpn_model_last_flops(const mpn_model *m, double *trunk_flops, double *head_f
   return MPN_OK;
 }
 
-int mpn_model_trunk_dev(mpn_model *m, const float *image_dev, int32_t H, int32_t W) {
+int mpn_model_trunk_batch_dev(mpn_model *m, const float *images_dev, int32_t N, int32_t H, int32_t W) {
   if (!m) return MPN_ERR_ARG;
   mpn_ctx *ctx = m->ctx;
   MPN_CUDA(ctx, cudaSetDevice(ctx->device));
-  MPN_CHECK_ARG(ctx, image_dev && H > 0 && W > 0 && H <= m->d.max_h && W <= m->d.max_w, "image missing or larger than max_h x max_w");
-  MPN_TRY(ensure_trunk(m, H, W));
-  return run_trunk(m, image_dev);
+  MPN_CHECK_ARG(ctx, N >= 1 && N <= MPN_MAX_BATCH, "batch size N must be in 1..MPN_MAX_BATCH");
+  MPN_CHECK_ARG(ctx, images_dev && H > 0 && W > 0 && H <= m->d.max_h && W <= m->d.max_w, "image missing or larger than max_h x max_w");
+  MPN_TRY(ensure_trunk(m, N, H, W));
+  return run_trunk(m, images_dev);
+}
+
+int mpn_model_trunk_dev(mpn_model *m, const float *image_dev, int32_t H, int32_t W) {
+  return mpn_model_trunk_batch_dev(m, image_dev, 1, H, W);
+}
+
+int mpn_model_trunk_batch(mpn_model *m, const float *images, int32_t N, int32_t H, int32_t W) {
+  if (!m) return MPN_ERR_ARG;
+  mpn_ctx *ctx = m->ctx;
+  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
+  MPN_CHECK_ARG(ctx, images && N >= 1 && N <= MPN_MAX_BATCH && H > 0 && W > 0, "images missing or batch size outside 1..MPN_MAX_BATCH");
+  const size_t bytes = sizeof(float) * 3 * (size_t)N * H * W;
+  MPN_TRY(m->image_dev.ensure(ctx, bytes));
+  MPN_CUDA(ctx, cudaMemcpyAsync(m->image_dev.p, images, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  MPN_TRY(mpn_model_trunk_batch_dev(m, (const float *)m->image_dev.p, N, H, W));
+  MPN_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return MPN_OK;
 }
 
 int mpn_model_trunk(mpn_model *m, const float *image, int32_t H, int32_t W) {
@@ -913,6 +936,129 @@ int mpn_model_detect_nms(mpn_model *m, const float *image, int32_t H, int32_t W,
   if (bboxes) MPN_CUDA(ctx, cudaMemcpyAsync(bboxes, m->bboxes_dev.p, sizeof(float) * (size_t)R * 4 * C, cudaMemcpyDeviceToHost, ctx->stream));
   if (keep_idx) MPN_CUDA(ctx, cudaMemcpyAsync(keep_idx, m->keep_idx_dev.p, sizeof(int32_t) * (size_t)(C - 1) * R, cudaMemcpyDeviceToHost, ctx->stream));
   if (keep_counts) MPN_CUDA(ctx, cudaMemcpyAsync(keep_counts, m->keep_counts_dev.p, sizeof(int32_t) * (size_t)(C - 1), cudaMemcpyDeviceToHost, ctx->stream));
+  MPN_TRY(mpn_ovf_copy_async(ctx, ctx->stream));
+  MPN_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return mpn_ovf_test(ctx);
+}
+
+// ---- N images in one pass: host-side validation of the batch description (nothing is launched before it passes)
+static int batch_desc(mpn_model *m, int32_t N, const int64_t *offs, const float *im_scale, const float *W0, const float *H0,
+                      MpnBatch &b, int &cap) {
+  mpn_ctx *ctx = m->ctx;
+  MPN_CHECK_ARG(ctx, N >= 1 && N <= MPN_MAX_BATCH, "batch size N must be in 1..MPN_MAX_BATCH");
+  MPN_CHECK_ARG(ctx, offs && im_scale && W0 && H0, "img_offsets / im_scale / W0 / H0 missing");
+  MPN_CHECK_ARG(ctx, offs[0] == 0, "img_offsets[0] must be 0");
+  memset(&b, 0, sizeof b);
+  b.n = N; cap = 0;
+  for (int i = 0; i < N; ++i) {
+    MPN_CHECK_ARG(ctx, offs[i + 1] - offs[i] >= 1, "every image needs at least one proposal (img_offsets strictly increasing)");
+    MPN_CHECK_ARG(ctx, offs[i + 1] <= m->d.max_rois, "R_total out of range (R_total <= max_rois)");
+    b.off[i] = (int)offs[i]; b.scale[i] = im_scale[i]; b.W0[i] = W0[i]; b.H0[i] = H0[i];
+    cap = std::max(cap, (int)(offs[i + 1] - offs[i]));
+  }
+  b.off[N] = (int)offs[N];
+  return MPN_OK;
+}
+
+// trunk over the batch, heads over all R_total rows, per-image clamp, gather + NMS over N x (C-1) segments of capacity `cap`
+// (segment i * (C-1) + j - 1 at sb / keep_idx_dev + seg * cap), one record per image into the sink. Results stay in the
+// model's buffers.
+static int detect_nms_batch_core(mpn_model *m, const float *images_dev, int32_t N, int32_t H, int32_t W, const float *boxes_dev,
+                                 const MpnBatch &b, int cap, float score_thresh, float nms_thr) {
+  mpn_ctx *ctx = m->ctx;
+  const int C = m->d.num_classes, K = (int)m->cls_heads.size();
+  const int64_t R = b.off[N];
+  const int nseg = N * (C - 1);
+  MPN_CHECK_ARG(ctx, !m->sink || m->sink_n + N <= m->sink_cap, "detection sink is full (mpn_model_set_detection_sink capacity)");
+  MPN_TRY(mpn_model_trunk_batch_dev(m, images_dev, N, H, W));
+  MPN_TRY(ensure_heads(m, R));
+  MPN_TRY(m->rois_dev.ensure(ctx, sizeof(float) * 5 * (size_t)R));
+  MPN_TRY(m->sb_dev.ensure(ctx, sizeof(float) * (size_t)nseg * cap * 5 + 256));
+  MPN_TRY(m->src_idx_dev.ensure(ctx, sizeof(int32_t) * (size_t)nseg * cap + 256));
+  MPN_TRY(m->counts_dev.ensure(ctx, sizeof(int32_t) * (size_t)nseg + 256));
+  MPN_TRY(m->keep_idx_dev.ensure(ctx, sizeof(int32_t) * (size_t)nseg * cap + 256));
+  MPN_TRY(m->keep_counts_dev.ensure(ctx, sizeof(int32_t) * (size_t)nseg + 256));
+  MPN_TRY(mpn_project_rois_batch_launch(ctx, boxes_dev, R, b, (float *)m->rois_dev.p));
+  MPN_TRY(run_heads(m, (const float *)m->rois_dev.p, R, /*apply_bbox_norm=*/false));
+  const int do_softmax = (K > 1) ? 1 : (m->d.no_softmax ? 0 : 1);
+  MPN_TRY(mpn_detect_tail_batch_launch(ctx, (const float *)m->cls_logits.p, R, C, K, do_softmax, (float *)m->scores_dev.p,
+                                       (const float *)m->bbox_raw.p, boxes_dev, b, (float *)m->bboxes_dev.p, m->d.has_bbox_norm ? 1 : 0,
+                                       m->d.bbox_mean, m->d.bbox_std));
+  MPN_TRY(mpn_gather_scored_batch_launch(ctx, (const float *)m->scores_dev.p, (const float *)m->bboxes_dev.p, C, score_thresh, b, cap,
+                                         (float *)m->sb_dev.p, (int32_t *)m->src_idx_dev.p, (int32_t *)m->counts_dev.p));
+  MPN_TRY(mpn_nms_launch(ctx, (const float *)m->sb_dev.p, cap, nseg, (const int32_t *)m->counts_dev.p, (const int32_t *)m->src_idx_dev.p,
+                         nms_thr, (int32_t *)m->keep_idx_dev.p, (int32_t *)m->keep_counts_dev.p));
+  if (m->sink) {
+    for (int i = 0; i < N; ++i) {
+      MPN_TRY(mpn_pack_detections_launch(ctx, (const float *)m->scores_dev.p + (size_t)b.off[i] * C,
+                                         (const float *)m->bboxes_dev.p + (size_t)b.off[i] * 4 * C, C,
+                                         (const int32_t *)m->keep_idx_dev.p + (size_t)i * (C - 1) * cap,
+                                         (const int32_t *)m->keep_counts_dev.p + (size_t)i * (C - 1), cap, m->sink_top_k,
+                                         m->sink + (size_t)m->sink_n * MPN_REC_FLOATS));
+      ++m->sink_n;
+    }
+  }
+  return MPN_OK;
+}
+
+// results of detect_nms_batch_core -> the caller's buffers (device or host, by `kind`): keep lists repacked from capacity
+// `cap` per segment to R_i per segment, image i's block at (C-1) * off[i]
+static int detect_nms_batch_copy_out(mpn_model *m, const MpnBatch &b, int cap, cudaMemcpyKind kind, float *scores, float *bboxes,
+                                     int32_t *keep_idx, int32_t *keep_counts) {
+  mpn_ctx *ctx = m->ctx;
+  const int C = m->d.num_classes, N = b.n;
+  const int64_t R = b.off[N];
+  if (scores) MPN_CUDA(ctx, cudaMemcpyAsync(scores, m->scores_dev.p, sizeof(float) * (size_t)R * C, kind, ctx->stream));
+  if (bboxes) MPN_CUDA(ctx, cudaMemcpyAsync(bboxes, m->bboxes_dev.p, sizeof(float) * (size_t)R * 4 * C, kind, ctx->stream));
+  if (keep_idx)
+    for (int i = 0; i < N; ++i) {
+      const size_t Ri = (size_t)(b.off[i + 1] - b.off[i]);
+      MPN_CUDA(ctx, cudaMemcpy2DAsync(keep_idx + (size_t)(C - 1) * b.off[i], sizeof(int32_t) * Ri,
+                                      (const int32_t *)m->keep_idx_dev.p + (size_t)i * (C - 1) * cap, sizeof(int32_t) * (size_t)cap,
+                                      sizeof(int32_t) * Ri, (size_t)(C - 1), kind, ctx->stream));
+    }
+  if (keep_counts)
+    MPN_CUDA(ctx, cudaMemcpyAsync(keep_counts, m->keep_counts_dev.p, sizeof(int32_t) * (size_t)N * (C - 1), kind, ctx->stream));
+  return MPN_OK;
+}
+
+int mpn_model_detect_nms_batch_dev(mpn_model *m, const float *images_dev, int32_t N, int32_t H, int32_t W, const float *boxes_dev,
+                                   const int64_t *img_offsets, const float *im_scale, const float *W0, const float *H0,
+                                   float score_thresh, float nms_thr, float *scores_dev, float *bboxes_dev, int32_t *keep_idx_dev,
+                                   int32_t *keep_counts_dev) {
+  if (!m) return MPN_ERR_ARG;
+  mpn_ctx *ctx = m->ctx;
+  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
+  MPN_CHECK_ARG(ctx, images_dev && boxes_dev, "images/boxes missing");
+  MpnBatch b; int cap = 0;
+  MPN_TRY(batch_desc(m, N, img_offsets, im_scale, W0, H0, b, cap));
+  if (N == 1)        // one image: the single-image path, byte for byte
+    return mpn_model_detect_nms_dev(m, images_dev, H, W, boxes_dev, img_offsets[1], im_scale[0], W0[0], H0[0], score_thresh, nms_thr,
+                                    scores_dev, bboxes_dev, keep_idx_dev, keep_counts_dev);
+  MPN_TRY(detect_nms_batch_core(m, images_dev, N, H, W, boxes_dev, b, cap, score_thresh, nms_thr));
+  return detect_nms_batch_copy_out(m, b, cap, cudaMemcpyDeviceToDevice, scores_dev, bboxes_dev, keep_idx_dev, keep_counts_dev);
+}
+
+int mpn_model_detect_nms_batch(mpn_model *m, const float *images, int32_t N, int32_t H, int32_t W, const float *boxes,
+                               const int64_t *img_offsets, const float *im_scale, const float *W0, const float *H0, float score_thresh,
+                               float nms_thr, float *scores, float *bboxes, int32_t *keep_idx, int32_t *keep_counts) {
+  if (!m) return MPN_ERR_ARG;
+  mpn_ctx *ctx = m->ctx;
+  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
+  MPN_CHECK_ARG(ctx, images && boxes && H > 0 && W > 0, "images/boxes missing");
+  MpnBatch b; int cap = 0;
+  MPN_TRY(batch_desc(m, N, img_offsets, im_scale, W0, H0, b, cap));
+  if (N == 1)
+    return mpn_model_detect_nms(m, images, H, W, boxes, img_offsets[1], im_scale[0], W0[0], H0[0], score_thresh, nms_thr, scores, bboxes,
+                                keep_idx, keep_counts);
+  const int64_t R = b.off[N];
+  const size_t bytes = sizeof(float) * 3 * (size_t)N * H * W;
+  MPN_TRY(m->image_dev.ensure(ctx, bytes));
+  MPN_TRY(m->boxes_dev.ensure(ctx, sizeof(float) * 4 * (size_t)R));
+  MPN_CUDA(ctx, cudaMemcpyAsync(m->image_dev.p, images, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  MPN_CUDA(ctx, cudaMemcpyAsync(m->boxes_dev.p, boxes, sizeof(float) * 4 * (size_t)R, cudaMemcpyHostToDevice, ctx->stream));
+  MPN_TRY(detect_nms_batch_core(m, (const float *)m->image_dev.p, N, H, W, (const float *)m->boxes_dev.p, b, cap, score_thresh, nms_thr));
+  MPN_TRY(detect_nms_batch_copy_out(m, b, cap, cudaMemcpyDeviceToHost, scores, bboxes, keep_idx, keep_counts));
   MPN_TRY(mpn_ovf_copy_async(ctx, ctx->stream));
   MPN_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return mpn_ovf_test(ctx);

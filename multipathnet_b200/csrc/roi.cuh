@@ -9,6 +9,8 @@ struct RoiJob {
   const float *lv[ROI_MAX_LEVELS];
   int nlev;                        // number of valid levels incl. level 0
   int H, W, C;
+  int nimg;                        // images in the pyramid (image stride H * W * C); a ROI naming another raises MPN_FLAG_BAD_BATCH
+  unsigned *flag;                  // the ctx's device flag word
   float scale;                     // spatial scale
   int region;                      // 0: ROI, 1..3: foveal x1.5, x2, x4
   __nv_bfloat16 *out_hi, *out_lo;  // R x bins x out_ld
