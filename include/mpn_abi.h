@@ -235,6 +235,19 @@ int mpn_get_images_u8(mpn_ctx *ctx, const uint8_t *im_hwc, int32_t H0, int32_t W
                       int32_t h, int32_t w, float *out);
 int mpn_get_images_u8_dev(mpn_ctx *ctx, const uint8_t *im_hwc_dev, int32_t H0, int32_t W0, const mpn_image_transform *tf,
                           int32_t h, int32_t w, float *out_dev);
+/* host-only (no GPU): getImages sizes of N images (mpn_get_images_size of each: h, w, im_scale arrays of N, any may be
+ * NULL) and the padded canvas H = max h_i, W = max w_i. Fails for N outside 1..MPN_MAX_BATCH or a size <= 0. */
+int mpn_get_images_batch_size(int32_t N, const int32_t *H0, const int32_t *W0, double scale, double max_size,
+                              int32_t *h, int32_t *w, double *im_scale, int32_t *H, int32_t *W);
+/* getImages of N raw images into one zero-padded N x 3 x H x W batch (ImageDetect.lua:44-50), in one launch. ims_hwc: the
+ * images' bytes back to back, image i H0[i] x W0[i] x 3 interleaved RGB at byte offset sum_{j<i} 3*H0[j]*W0[j]; one
+ * transformer for all. Image i's block [0,h_i) x [0,w_i) is exactly what mpn_get_images_u8 gives for it alone, every other
+ * element is +0.0f (written by the kernel: out needs no clearing). H, W as mpn_get_images_batch_size, H <= 65535.
+ * Host buffers, synchronous; _dev: device buffers, stream-ordered. */
+int mpn_get_images_batch_u8(mpn_ctx *ctx, const uint8_t *ims_hwc, int32_t N, const int32_t *H0, const int32_t *W0,
+                            const mpn_image_transform *tf, double scale, double max_size, float *out);
+int mpn_get_images_batch_u8_dev(mpn_ctx *ctx, const uint8_t *ims_hwc_dev, int32_t N, const int32_t *H0, const int32_t *W0,
+                                const mpn_image_transform *tf, double scale, double max_size, float *out_dev);
 /* getImages + model:get(1):forward: uploads the RAW image (host), transforms and scales it on the device into the
  * model's image buffer and runs the trunk; *im_scale, *h, *w as mpn_get_images_size. Follow with mpn_model_detect(...,
  * image = NULL, recompute_features = 0) on the cached features. */
@@ -284,6 +297,21 @@ int mpn_model_detect_nms_submit_u8(mpn_model *m, const uint8_t *im_hwc, int32_t 
                                    const mpn_image_transform *tf, double scale, double max_size, const float *boxes,
                                    int64_t R, float score_thresh, float nms_thr, float *scores, float *bboxes,
                                    int32_t *keep_idx, int32_t *keep_counts, int32_t *ticket);
+/* Pipelined mpn_model_detect_nms_batch from N RAW images of any sizes (packed as mpn_get_images_batch_u8): the packed bytes
+ * and the boxes cross the bus on the copy stream, getImages pads the images into one canvas (H = max h_i, W = max w_i) on
+ * the device, and the batched trunk, heads and NMS follow. boxes R_total x 4 in each image's ORIGINAL coordinates, image i
+ * owning rows [img_offsets[i], img_offsets[i+1]); each image is projected with its own im_scale_i (as float) and clamped
+ * to its own W0[i] x H0[i]. Outputs, their layout and the detection sink (N records in image order) as
+ * mpn_model_detect_nms_batch. Same ticket protocol and the same two slots as mpn_model_detect_nms_submit(_u8): the kinds
+ * may be interleaved, and mpn_model_detect_nms_wait completes either. N = 1 is exactly mpn_model_detect_nms_submit_u8.
+ * A canvas that differs from the previous call's re-plans the trunk. Every argument is checked before anything is
+ * enqueued: 1 <= N <= MPN_MAX_BATCH, H0, W0 > 0, canvas within the model's max_h x max_w, every R_i >= 1,
+ * R_total <= max_rois, swap entries 1..3, pointers present. The synchronous form is submit + wait; device-resident callers
+ * compose mpn_get_images_batch_u8_dev with mpn_model_detect_nms_batch_dev. */
+int mpn_model_detect_nms_batch_submit_u8(mpn_model *m, const uint8_t *ims_hwc, int32_t N, const int32_t *H0, const int32_t *W0,
+                                         const mpn_image_transform *tf, double scale, double max_size,
+                                         const float *boxes, const int64_t *img_offsets, float score_thresh, float nms_thr,
+                                         float *scores, float *bboxes, int32_t *keep_idx, int32_t *keep_counts, int32_t *ticket);
 int mpn_model_detect_nms_wait(mpn_model *m, int32_t ticket);
 /* Tester_FRCNN:testOne with its test-time options (Tester_FRCNN.lua:54-139) in one stream-ordered pass, nothing but the
  * inputs and the final results crossing the bus: pass 1 = detect on the proposals, clamped to the image (:72-78); passes

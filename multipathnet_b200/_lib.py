@@ -120,6 +120,12 @@ SIGNATURES = {
     "mpn_get_images_dev": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, _vp, C.c_int32, C.c_int32, _vp]),
     "mpn_get_images_u8": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, _vp, C.c_int32, C.c_int32, _vp]),
     "mpn_get_images_u8_dev": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, _vp, C.c_int32, C.c_int32, _vp]),
+    "mpn_get_images_batch_size": (C.c_int, [C.c_int32, _i32p, _i32p, C.c_double, C.c_double, _i32p, _i32p, C.POINTER(C.c_double), _i32p,
+                                            _i32p]),
+    "mpn_get_images_batch_u8": (C.c_int, [_vp, _vp, C.c_int32, _i32p, _i32p, _vp, C.c_double, C.c_double, _vp]),
+    "mpn_get_images_batch_u8_dev": (C.c_int, [_vp, _vp, C.c_int32, _i32p, _i32p, _vp, C.c_double, C.c_double, _vp]),
+    "mpn_model_detect_nms_batch_submit_u8": (C.c_int, [_vp, _vp, C.c_int32, _i32p, _i32p, _vp, C.c_double, C.c_double, _vp, _i64p, C.c_float,
+                                                       C.c_float, _vp, _vp, _vp, _vp, _i32p]),
     "mpn_model_detect_nms_submit_u8": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, _vp, C.c_double, C.c_double, _vp, C.c_int64, C.c_float, C.c_float,
                                                  _vp, _vp, _vp, _vp, _i32p]),
     "mpn_model_trunk_image": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, _vp, C.c_double, C.c_double, C.POINTER(C.c_double), _i32p, _i32p]),
@@ -210,6 +216,29 @@ def _ptr(a) -> Optional[int]:
 
 def _f32(a) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.float32)
+
+
+def _raw_batch(ims, scale: float, max_size: float):
+    """host-side checks of N raw images for the batched getImages -> (list of contiguous H0 x W0 x 3 uint8 arrays,
+    H0 int32 N, W0 int32 N, [(h_i, w_i, im_scale_i)], canvas (H, W)); raises ValueError before any library call. The sizes
+    follow image_detect's rule, which tests/test_batch_raw_cpu.py pins to mpn_get_images_batch_size."""
+    from .image_detect import _get_images_size
+    if not isinstance(ims, (list, tuple)) or not 1 <= len(ims) <= MPN_MAX_BATCH:
+        raise ValueError(f"expected a list of 1..{MPN_MAX_BATCH} raw images")
+    out = []
+    for i, im in enumerate(ims):
+        if not isinstance(im, np.ndarray) or im.dtype != np.uint8 or im.ndim != 3 or im.shape[2] != 3 or im.shape[0] < 1 or im.shape[1] < 1:
+            raise ValueError(f"image {i}: expected an H0 x W0 x 3 uint8 array")
+        out.append(np.ascontiguousarray(im))
+    if not (scale > 0 and max_size > 0):
+        raise ValueError("scale and max_size must be > 0")
+    H0 = np.array([im.shape[0] for im in out], np.int32)
+    W0 = np.array([im.shape[1] for im in out], np.int32)
+    sizes = [_get_images_size(int(h), int(w), scale, max_size) for h, w in zip(H0, W0)]
+    H, W = max(h for h, _, _ in sizes), max(w for _, w, _ in sizes)
+    if min(min(h, w) for h, w, _ in sizes) < 1 or H > 65535:
+        raise ValueError(f"scaled sizes out of range: canvas {H} x {W}")
+    return out, H0, W0, sizes, (H, W)
 
 
 class Context:
@@ -418,6 +447,17 @@ class Context:
                    "mpn_get_images_u8")
         return out, float(s.value)
 
+    def get_images_batch_u8(self, ims, kind: str, scale: float = 600, max_size: float = 1000):
+        """getImages of N raw H0 x W0 x 3 uint8 images of any sizes into one zero-padded canvas on the device (one launch)
+        -> (batch N x 3 x H x W, [im_scale_i], [(h_i, w_i)]); image i fills [0, h_i) x [0, w_i) of its plane, the rest is 0"""
+        ims, H0, W0, sizes, (H, W) = _raw_batch(ims, scale, max_size)
+        tf = CImageTransform.of(kind)
+        raw = np.concatenate([im.reshape(-1) for im in ims])
+        out = np.empty((len(ims), 3, H, W), np.float32)
+        self.check(self.lib.mpn_get_images_batch_u8(self.h, _ptr(raw), len(ims), H0.ctypes.data_as(_i32p), W0.ctypes.data_as(_i32p),
+                                                    C.addressof(tf), float(scale), float(max_size), _ptr(out)), "mpn_get_images_batch_u8")
+        return out, [s for _, _, s in sizes], [(h, w) for h, w, _ in sizes]
+
     def bbox_norm(self, deltas, mean, std) -> np.ndarray:
         d = _f32(deltas).copy()
         m, s = _f32(mean).reshape(4), _f32(std).reshape(4)
@@ -590,6 +630,7 @@ class Model:
         self.h = h
         self.C = spec.num_classes
         self.max_rois = int(max_rois)
+        self.max_h, self.max_w = int(max_h), int(max_w)
         self._trunk_n = 1                  # images of the last trunk forward (the leading size of trunk_slot)
         import weakref
         ctx._models.append(weakref.ref(self))
@@ -752,10 +793,51 @@ class Model:
         self._inflight[t.value] = out
         return t.value
 
+    def detect_nms_batch_submit_u8(self, ims, boxes_list, kind: str, scale: float = 600, max_size: float = 1000,
+                                   score_thresh: float = -1.5, nms_thr: float = 0.3):
+        """pipelined detect_nms_batch from N RAW uint8 H0 x W0 x 3 images of any sizes (mpn_model_detect_nms_batch_submit_u8):
+        getImages pads them into one canvas on the device. boxes_list[i]: R_i x 4 in image i's ORIGINAL coordinates.
+        Returns a ticket; detect_nms_wait(ticket) returns one (scores, bboxes, keeps) per image, as detect_nms_batch."""
+        ims, H0, W0, sizes, (H, W) = _raw_batch(ims, scale, max_size)
+        N = len(ims)
+        if len(boxes_list) != N:
+            raise ValueError(f"{N} images need {N} box arrays, got {len(boxes_list)}")
+        boxes = [_f32(b) for b in boxes_list]
+        if any(b.ndim != 2 or b.shape[1] != 4 for b in boxes):
+            raise ValueError("every box array must be R_i x 4")
+        if H > self.max_h or W > self.max_w:
+            raise ValueError(f"padded canvas {H} x {W} larger than the model's max_h x max_w = {self.max_h} x {self.max_w}")
+        offs, _, _, _ = self._batch_args(N, [b.shape[0] for b in boxes], [s for _, _, s in sizes], [(int(w), int(h)) for h, w in zip(H0, W0)])
+        Rt, Cn = int(offs[-1]), self.C
+        out = dict(im=np.concatenate([im.reshape(-1) for im in ims]), b=np.ascontiguousarray(np.concatenate(boxes, 0)), H0=H0, W0=W0,
+                   offs=offs, scores=np.empty((Rt, Cn), np.float32), bboxes=np.empty((Rt, 4 * Cn), np.float32),
+                   keep=np.empty((Cn - 1) * Rt, np.int32), counts=np.empty((N, Cn - 1), np.int32), tf=CImageTransform.of(kind))
+        t = C.c_int32(-1)
+        self._trunk_n = N
+        self.ctx.check(self.ctx.lib.mpn_model_detect_nms_batch_submit_u8(
+            self.h, _ptr(out["im"]), N, H0.ctypes.data_as(_i32p), W0.ctypes.data_as(_i32p), C.addressof(out["tf"]), float(scale),
+            float(max_size), _ptr(out["b"]), offs.ctypes.data_as(_i64p), float(score_thresh), float(nms_thr), _ptr(out["scores"]),
+            _ptr(out["bboxes"]), _ptr(out["keep"]), _ptr(out["counts"]), C.byref(t)), "mpn_model_detect_nms_batch_submit_u8")
+        self._inflight = getattr(self, "_inflight", {})
+        self._inflight[t.value] = out
+        return t.value
+
     def detect_nms_wait(self, ticket: int):
+        """results of a submission: (scores, bboxes, keeps) for a single image, one such tuple per image for a batch"""
         self.ctx.check(self.ctx.lib.mpn_model_detect_nms_wait(self.h, int(ticket)), "mpn_model_detect_nms_wait")
         o = self._inflight.pop(ticket)
+        if "offs" in o:
+            return self._split_batch(o["offs"], o["scores"], o["bboxes"], o["keep"], o["counts"])
         return o["scores"], o["bboxes"], [o["keep"][j, : o["counts"][j]].copy() for j in range(self.C - 1)]
+
+    def _split_batch(self, offs, scores, bboxes, keep, counts):
+        """the flat outputs of a batch call -> [(scores R_i x C, bboxes R_i x 4C, [keep rows per class])] per image"""
+        Cn, out = self.C, []
+        for i in range(len(offs) - 1):
+            r0, r1 = int(offs[i]), int(offs[i + 1])
+            k = keep[(Cn - 1) * r0:(Cn - 1) * r1].reshape(Cn - 1, r1 - r0)
+            out.append((scores[r0:r1], bboxes[r0:r1], [k[j, :counts[i, j]].copy() for j in range(Cn - 1)]))
+        return out
 
     def detect_nms_dev(self, image_dev, H: int, W: int, boxes_dev, R: int, im_scale: float, W0: float, H0: float,
                        score_thresh: float, nms_thr: float, scores_dev=None, bboxes_dev=None, keep_idx_dev=None,
@@ -800,12 +882,7 @@ class Model:
         self.ctx.check(self.ctx.lib.mpn_model_detect_nms_batch(
             self.h, _ptr(im), N, im.shape[2], im.shape[3], _ptr(b), offs.ctypes.data_as(_i64p), _ptr(sc), _ptr(w0), _ptr(h0),
             float(score_thresh), float(nms_thr), _ptr(scores), _ptr(bboxes), _ptr(keep), _ptr(counts)), "mpn_model_detect_nms_batch")
-        out = []
-        for i in range(N):
-            r0, r1 = int(offs[i]), int(offs[i + 1])
-            k = keep[(Cn - 1) * r0:(Cn - 1) * r1].reshape(Cn - 1, r1 - r0)
-            out.append((scores[r0:r1], bboxes[r0:r1], [k[j, :counts[i, j]].copy() for j in range(Cn - 1)]))
-        return out
+        return self._split_batch(offs, scores, bboxes, keep, counts)
 
     def detect_nms_batch_dev(self, images_dev, N: int, H: int, W: int, boxes_dev, R_list: Sequence[int], im_scales, sizes,
                              score_thresh: float, nms_thr: float, scores_dev=None, bboxes_dev=None, keep_idx_dev=None,

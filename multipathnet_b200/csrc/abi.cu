@@ -18,6 +18,12 @@ int mpn_context_region_launch(mpn_ctx *, const float *, int64_t, float, float *)
 int mpn_get_images_launch(mpn_ctx *, const float *, int32_t, int32_t, const mpn_image_transform *, int32_t, int32_t, float *);
 int mpn_get_images_size_impl(int32_t, int32_t, double, double, int32_t *, int32_t *, double *);
 int mpn_get_images_u8_launch(mpn_ctx *, const uint8_t *, int32_t, int32_t, const mpn_image_transform *, int32_t, int32_t, float *);
+int mpn_get_images_batch_size_impl(int32_t, const int32_t *, const int32_t *, double, double, int32_t *, int32_t *, double *, int32_t *,
+                                   int32_t *);
+int mpn_get_images_batch_launch(mpn_ctx *, const float *, const uint8_t *, int32_t, const int32_t *, const int32_t *, const int32_t *,
+                                const int32_t *, int32_t, int32_t, const mpn_image_transform *, float *);
+int mpn_get_images_batch_check(mpn_ctx *, int32_t, const int32_t *, const int32_t *, const mpn_image_transform *, double, double, int32_t *,
+                               int32_t *, double *, int32_t &, int32_t &, size_t &);
 int mpn_bbox_norm_launch(mpn_ctx *, float *, int64_t, int64_t, const float *, const float *);
 int mpn_bbox_decode_launch(mpn_ctx *, const float *, const float *, int64_t, int, int, float, float, float *);
 int mpn_split_rows_launch(mpn_ctx *, const float *, int64_t, int64_t, int64_t, __nv_bfloat16 *, __nv_bfloat16 *, int64_t);
@@ -513,6 +519,36 @@ int mpn_get_images_u8(mpn_ctx *ctx, const uint8_t *im_hwc, int32_t H0, int32_t W
   MPN_TRY(a.commit());
   MPN_CUDA(ctx, cudaMemcpyAsync(a.at<uint8_t>(o_i), im_hwc, bi, cudaMemcpyHostToDevice, ctx->stream));
   MPN_TRY(mpn_get_images_u8_launch(ctx, a.at<uint8_t>(o_i), H0, W0, tf, h, w, a.at<float>(o_o)));
+  MPN_CUDA(ctx, cudaMemcpyAsync(out, a.at<float>(o_o), bo, cudaMemcpyDeviceToHost, ctx->stream));
+  MPN_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return MPN_OK;
+}
+int mpn_get_images_batch_size(int32_t N, const int32_t *H0, const int32_t *W0, double scale, double max_size, int32_t *h, int32_t *w,
+                              double *im_scale, int32_t *H, int32_t *W) {
+  return mpn_get_images_batch_size_impl(N, H0, W0, scale, max_size, h, w, im_scale, H, W);
+}
+int mpn_get_images_batch_u8_dev(mpn_ctx *ctx, const uint8_t *ims_hwc_dev, int32_t N, const int32_t *H0, const int32_t *W0,
+                                const mpn_image_transform *tf, double scale, double max_size, float *out_dev) {
+  if (!ctx) return MPN_ERR_ARG;
+  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
+  MPN_CHECK_ARG(ctx, ims_hwc_dev && out_dev, "getImages: buffers missing");
+  int32_t h[MPN_MAX_BATCH], w[MPN_MAX_BATCH], H = 0, W = 0; size_t bi = 0;
+  MPN_TRY(mpn_get_images_batch_check(ctx, N, H0, W0, tf, scale, max_size, h, w, nullptr, H, W, bi));
+  return mpn_get_images_batch_launch(ctx, nullptr, ims_hwc_dev, N, H0, W0, h, w, H, W, tf, out_dev);
+}
+int mpn_get_images_batch_u8(mpn_ctx *ctx, const uint8_t *ims_hwc, int32_t N, const int32_t *H0, const int32_t *W0,
+                            const mpn_image_transform *tf, double scale, double max_size, float *out) {
+  if (!ctx) return MPN_ERR_ARG;
+  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
+  MPN_CHECK_ARG(ctx, ims_hwc && out, "getImages: buffers missing");
+  int32_t h[MPN_MAX_BATCH], w[MPN_MAX_BATCH], H = 0, W = 0; size_t bi = 0;
+  MPN_TRY(mpn_get_images_batch_check(ctx, N, H0, W0, tf, scale, max_size, h, w, nullptr, H, W, bi));
+  Arena a{ctx};
+  const size_t bo = sizeof(float) * 3 * (size_t)N * H * W;
+  size_t o_i = a.reserve(bi), o_o = a.reserve(bo);
+  MPN_TRY(a.commit());
+  MPN_CUDA(ctx, cudaMemcpyAsync(a.at<uint8_t>(o_i), ims_hwc, bi, cudaMemcpyHostToDevice, ctx->stream));
+  MPN_TRY(mpn_get_images_batch_launch(ctx, nullptr, a.at<uint8_t>(o_i), N, H0, W0, h, w, H, W, tf, a.at<float>(o_o)));
   MPN_CUDA(ctx, cudaMemcpyAsync(out, a.at<float>(o_o), bo, cudaMemcpyDeviceToHost, ctx->stream));
   MPN_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return MPN_OK;

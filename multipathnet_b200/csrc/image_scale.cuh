@@ -163,4 +163,31 @@ MPN_HD float scaled_pixel(const TransformedImage &I, int h, int w, int c, int y,
   return scaled_pixel(I, h, w, c, y, x, axis_scale(I.W0, w), axis_scale(I.H0, h));
 }
 
+// getImages of N images into one zero-padded N x 3 x H x W canvas (ImageDetect.lua:44-50: images:resize(n,3,maxH,maxW):zero(),
+// each image copied top-left). The sources lie back to back: image n starts src_off elements after the shared base pointer
+// (3*H0*W0 per image, bytes for the uint8 source, floats for the fp32 one).
+enum { kMaxBatchImages = 64 };       // MPN_MAX_BATCH (include/mpn_abi.h)
+struct BatchImage {
+  int64_t src_off;
+  int32_t H0, W0;        // original size
+  int32_t h, w;          // scaled size (mpn_get_images_size)
+  float sx, sy;          // axis_scale(W0, w), axis_scale(H0, h), divided on the host
+};
+struct ImageBatch {
+  TransformedImage I;    // base pointer(s), byte table and transformer shared by all images; I.H0 / I.W0 unused
+  int32_t n, H, W;       // images, canvas
+  BatchImage img[kMaxBatchImages];
+};
+
+// element (n, c, y, x) of the canvas: image n's scaled pixel inside [0, h) x [0, w), +0.0f elsewhere
+MPN_HD float batch_pixel(const ImageBatch &B, int n, int c, int y, int x) {
+  const BatchImage &b = B.img[n];
+  if (y >= b.h || x >= b.w) return 0.0f;
+  TransformedImage I = B.I;
+  I.H0 = b.H0; I.W0 = b.W0;
+  if (I.im) I.im += b.src_off;
+  else I.im_u8 += b.src_off;
+  return scaled_pixel(I, b.h, b.w, c, y, x, b.sx, b.sy);
+}
+
 }  // namespace mpn_img

@@ -28,6 +28,10 @@ int mpn_gather_scored_batch_launch(mpn_ctx *, const float *, const float *, int,
 int mpn_get_images_launch(mpn_ctx *, const float *, int32_t, int32_t, const mpn_image_transform *, int32_t, int32_t, float *);
 int mpn_get_images_size_impl(int32_t, int32_t, double, double, int32_t *, int32_t *, double *);
 int mpn_get_images_u8_launch(mpn_ctx *, const uint8_t *, int32_t, int32_t, const mpn_image_transform *, int32_t, int32_t, float *);
+int mpn_get_images_batch_launch(mpn_ctx *, const float *, const uint8_t *, int32_t, const int32_t *, const int32_t *, const int32_t *,
+                                const int32_t *, int32_t, int32_t, const mpn_image_transform *, float *);
+int mpn_get_images_batch_check(mpn_ctx *, int32_t, const int32_t *, const int32_t *, const mpn_image_transform *, double, double, int32_t *,
+                               int32_t *, double *, int32_t &, int32_t &, size_t &);
 int mpn_bbox_norm_launch(mpn_ctx *, float *, int64_t, int64_t, const float *, const float *);
 int mpn_bbox_decode_launch(mpn_ctx *, const float *, const float *, int64_t, int, int, float, float, float *);
 int mpn_softmax_mean_launch(mpn_ctx *, const float *, int64_t, int, int, int, float *);
@@ -1064,16 +1068,9 @@ int mpn_model_detect_nms_batch(mpn_model *m, const float *images, int32_t N, int
   return mpn_ovf_test(ctx);
 }
 
-// image != null: the transformed + scaled fp32 image (H x W); else raw_u8: the RAW H0 x W0 x 3 byte image, transformed and
-// scaled on the device (get_images_kernel) to the size getImages prescribes
-static int submit_common(mpn_model *m, const float *image, int32_t H, int32_t W, const uint8_t *raw_u8, int32_t H0r, int32_t W0r,
-                         const mpn_image_transform *tf, double scale, double max_size, const float *boxes, int64_t R, float im_scale,
-                         float W0, float H0, float score_thresh, float nms_thr, float *scores, float *bboxes, int32_t *keep_idx,
-                         int32_t *keep_counts, int32_t *ticket) {
+// the pipeline slot the next ticket uses (its copy streams and events created on first use); fails while it is in flight
+static int pipe_slot(mpn_model *m, mpn_model::PipeSlot *&slot) {
   mpn_ctx *ctx = m->ctx;
-  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
-  MPN_CHECK_ARG(ctx, (image || raw_u8) && boxes && R > 0 && ticket, "image/boxes/ticket missing");
-  const int C = m->d.num_classes;
   mpn_model::PipeSlot &q = m->pipe[m->next_ticket & 1];
   if (q.busy) return mpn_fail(ctx, MPN_ERR_STATE, "two submissions are already in flight: call mpn_model_detect_nms_wait first");
   if (!m->s_h2d) {
@@ -1085,6 +1082,43 @@ static int submit_common(mpn_model *m, const float *image, int32_t H, int32_t W,
     MPN_CUDA(ctx, cudaEventCreateWithFlags(&q.compute, cudaEventDisableTiming));
     MPN_CUDA(ctx, cudaEventCreateWithFlags(&q.done, cudaEventDisableTiming));
   }
+  slot = &q;
+  return MPN_OK;
+}
+
+// after the slot's kernels: its private outputs (R rows, n_img x (C-1) keep counts) -> the caller's host buffers on the
+// device->host stream; the slot is in flight until mpn_model_detect_nms_wait(*ticket)
+static int pipe_finish(mpn_model *m, mpn_model::PipeSlot &q, int64_t R, int n_img, float *scores, float *bboxes, int32_t *keep_idx,
+                       int32_t *keep_counts, int32_t *ticket) {
+  mpn_ctx *ctx = m->ctx;
+  const int C = m->d.num_classes;
+  MPN_CUDA(ctx, cudaEventRecord(q.compute, ctx->stream));
+  MPN_CUDA(ctx, cudaStreamWaitEvent(m->s_d2h, q.compute, 0));
+  if (scores) MPN_CUDA(ctx, cudaMemcpyAsync(scores, q.scores.p, sizeof(float) * (size_t)R * C, cudaMemcpyDeviceToHost, m->s_d2h));
+  if (bboxes) MPN_CUDA(ctx, cudaMemcpyAsync(bboxes, q.bboxes.p, sizeof(float) * (size_t)R * 4 * C, cudaMemcpyDeviceToHost, m->s_d2h));
+  if (keep_idx) MPN_CUDA(ctx, cudaMemcpyAsync(keep_idx, q.keep_idx.p, sizeof(int32_t) * (size_t)(C - 1) * R, cudaMemcpyDeviceToHost, m->s_d2h));
+  if (keep_counts)
+    MPN_CUDA(ctx, cudaMemcpyAsync(keep_counts, q.keep_counts.p, sizeof(int32_t) * (size_t)n_img * (C - 1), cudaMemcpyDeviceToHost, m->s_d2h));
+  MPN_TRY(mpn_ovf_copy_async(ctx, m->s_d2h));
+  MPN_CUDA(ctx, cudaEventRecord(q.done, m->s_d2h));
+  q.busy = true; q.ticket = m->next_ticket;
+  *ticket = m->next_ticket++;
+  return MPN_OK;
+}
+
+// image != null: the transformed + scaled fp32 image (H x W); else raw_u8: the RAW H0 x W0 x 3 byte image, transformed and
+// scaled on the device (get_images_kernel) to the size getImages prescribes
+static int submit_common(mpn_model *m, const float *image, int32_t H, int32_t W, const uint8_t *raw_u8, int32_t H0r, int32_t W0r,
+                         const mpn_image_transform *tf, double scale, double max_size, const float *boxes, int64_t R, float im_scale,
+                         float W0, float H0, float score_thresh, float nms_thr, float *scores, float *bboxes, int32_t *keep_idx,
+                         int32_t *keep_counts, int32_t *ticket) {
+  mpn_ctx *ctx = m->ctx;
+  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
+  MPN_CHECK_ARG(ctx, (image || raw_u8) && boxes && R > 0 && ticket, "image/boxes/ticket missing");
+  const int C = m->d.num_classes;
+  mpn_model::PipeSlot *qp = nullptr;
+  MPN_TRY(pipe_slot(m, qp));
+  mpn_model::PipeSlot &q = *qp;
   if (raw_u8) {
     MPN_CHECK_ARG(ctx, tf && H0r > 0 && W0r > 0, "raw image: transformer / size missing");
     double s = 0;
@@ -1113,17 +1147,7 @@ static int submit_common(mpn_model *m, const float *image, int32_t H, int32_t W,
   MPN_TRY(mpn_model_detect_nms_dev(m, (const float *)q.image.p, H, W, (const float *)q.boxes.p, R, im_scale, W0, H0, score_thresh,
                                    nms_thr, scores ? (float *)q.scores.p : nullptr, bboxes ? (float *)q.bboxes.p : nullptr,
                                    keep_idx ? (int32_t *)q.keep_idx.p : nullptr, keep_counts ? (int32_t *)q.keep_counts.p : nullptr));
-  MPN_CUDA(ctx, cudaEventRecord(q.compute, ctx->stream));
-  MPN_CUDA(ctx, cudaStreamWaitEvent(m->s_d2h, q.compute, 0));
-  if (scores) MPN_CUDA(ctx, cudaMemcpyAsync(scores, q.scores.p, sizeof(float) * (size_t)R * C, cudaMemcpyDeviceToHost, m->s_d2h));
-  if (bboxes) MPN_CUDA(ctx, cudaMemcpyAsync(bboxes, q.bboxes.p, sizeof(float) * (size_t)R * 4 * C, cudaMemcpyDeviceToHost, m->s_d2h));
-  if (keep_idx) MPN_CUDA(ctx, cudaMemcpyAsync(keep_idx, q.keep_idx.p, sizeof(int32_t) * (size_t)(C - 1) * R, cudaMemcpyDeviceToHost, m->s_d2h));
-  if (keep_counts) MPN_CUDA(ctx, cudaMemcpyAsync(keep_counts, q.keep_counts.p, sizeof(int32_t) * (size_t)(C - 1), cudaMemcpyDeviceToHost, m->s_d2h));
-  MPN_TRY(mpn_ovf_copy_async(ctx, m->s_d2h));
-  MPN_CUDA(ctx, cudaEventRecord(q.done, m->s_d2h));
-  q.busy = true; q.ticket = m->next_ticket;
-  *ticket = m->next_ticket++;
-  return MPN_OK;
+  return pipe_finish(m, q, R, 1, scores, bboxes, keep_idx, keep_counts, ticket);
 }
 
 int mpn_model_detect_nms_submit(mpn_model *m, const float *image, int32_t H, int32_t W, const float *boxes, int64_t R,
@@ -1142,6 +1166,51 @@ int mpn_model_detect_nms_submit_u8(mpn_model *m, const uint8_t *im_hwc, int32_t 
   MPN_CHECK_ARG(m->ctx, im_hwc, "image missing");
   return submit_common(m, nullptr, 0, 0, im_hwc, H0, W0, tf, scale, max_size, boxes, R, 0.f, 0.f, 0.f, score_thresh, nms_thr, scores, bboxes,
                        keep_idx, keep_counts, ticket);
+}
+
+int mpn_model_detect_nms_batch_submit_u8(mpn_model *m, const uint8_t *ims_hwc, int32_t N, const int32_t *H0, const int32_t *W0,
+                                         const mpn_image_transform *tf, double scale, double max_size, const float *boxes,
+                                         const int64_t *img_offsets, float score_thresh, float nms_thr, float *scores, float *bboxes,
+                                         int32_t *keep_idx, int32_t *keep_counts, int32_t *ticket) {
+  if (!m) return MPN_ERR_ARG;
+  mpn_ctx *ctx = m->ctx;
+  MPN_CUDA(ctx, cudaSetDevice(ctx->device));
+  // every check on the host, before anything is enqueued
+  MPN_CHECK_ARG(ctx, N >= 1 && N <= MPN_MAX_BATCH, "batch size N must be in 1..MPN_MAX_BATCH");
+  MPN_CHECK_ARG(ctx, ims_hwc && H0 && W0 && tf && boxes && img_offsets && ticket, "images / H0 / W0 / transformer / boxes / img_offsets / ticket missing");
+  int32_t h[MPN_MAX_BATCH], w[MPN_MAX_BATCH], H = 0, W = 0; double s[MPN_MAX_BATCH]; size_t raw_bytes = 0;
+  MPN_TRY(mpn_get_images_batch_check(ctx, N, H0, W0, tf, scale, max_size, h, w, s, H, W, raw_bytes));
+  MPN_CHECK_ARG(ctx, H <= m->d.max_h && W <= m->d.max_w, "padded canvas larger than max_h x max_w");
+  float sc[MPN_MAX_BATCH], w0[MPN_MAX_BATCH], h0[MPN_MAX_BATCH];
+  for (int i = 0; i < N; ++i) { sc[i] = (float)s[i]; w0[i] = (float)W0[i]; h0[i] = (float)H0[i]; }   // as submit_common
+  MpnBatch b; int cap = 0;
+  MPN_TRY(batch_desc(m, N, img_offsets, sc, w0, h0, b, cap));
+  MPN_CHECK_ARG(ctx, !m->sink || m->sink_n + N <= m->sink_cap, "detection sink is full (mpn_model_set_detection_sink capacity)");
+  if (N == 1)        // one image: the single-image raw path, byte for byte
+    return submit_common(m, nullptr, 0, 0, ims_hwc, H0[0], W0[0], tf, scale, max_size, boxes, img_offsets[1], 0.f, 0.f, 0.f, score_thresh,
+                         nms_thr, scores, bboxes, keep_idx, keep_counts, ticket);
+  mpn_model::PipeSlot *qp = nullptr;
+  MPN_TRY(pipe_slot(m, qp));
+  mpn_model::PipeSlot &q = *qp;
+  const int C = m->d.num_classes;
+  const int64_t R = b.off[N];
+  MPN_TRY(q.image.ensure(ctx, sizeof(float) * 3 * (size_t)N * H * W));
+  MPN_TRY(q.raw_u8.ensure(ctx, raw_bytes));
+  MPN_TRY(q.boxes.ensure(ctx, sizeof(float) * 4 * (size_t)R));
+  MPN_TRY(q.scores.ensure(ctx, sizeof(float) * (size_t)R * C));
+  MPN_TRY(q.bboxes.ensure(ctx, sizeof(float) * (size_t)R * 4 * C));
+  MPN_TRY(q.keep_idx.ensure(ctx, sizeof(int32_t) * (size_t)(C - 1) * R));
+  MPN_TRY(q.keep_counts.ensure(ctx, sizeof(int32_t) * (size_t)N * (C - 1)));
+  MPN_CUDA(ctx, cudaMemcpyAsync(q.raw_u8.p, ims_hwc, raw_bytes, cudaMemcpyHostToDevice, m->s_h2d));
+  MPN_CUDA(ctx, cudaMemcpyAsync(q.boxes.p, boxes, sizeof(float) * 4 * (size_t)R, cudaMemcpyHostToDevice, m->s_h2d));
+  MPN_CUDA(ctx, cudaEventRecord(q.h2d, m->s_h2d));
+  MPN_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, q.h2d, 0));
+  MPN_TRY(mpn_get_images_batch_launch(ctx, nullptr, (const uint8_t *)q.raw_u8.p, N, H0, W0, h, w, H, W, tf, (float *)q.image.p));
+  MPN_TRY(detect_nms_batch_core(m, (const float *)q.image.p, N, H, W, (const float *)q.boxes.p, b, cap, score_thresh, nms_thr));
+  MPN_TRY(detect_nms_batch_copy_out(m, b, cap, cudaMemcpyDeviceToDevice, scores ? (float *)q.scores.p : nullptr,
+                                    bboxes ? (float *)q.bboxes.p : nullptr, keep_idx ? (int32_t *)q.keep_idx.p : nullptr,
+                                    keep_counts ? (int32_t *)q.keep_counts.p : nullptr));
+  return pipe_finish(m, q, R, N, scores, bboxes, keep_idx, keep_counts, ticket);
 }
 
 int mpn_model_detect_nms_wait(mpn_model *m, int32_t ticket) {
